@@ -25,6 +25,10 @@ and checked in `secondary.tp`.
 `--impl reference` times the reference's own CPU implementation of the path on the host cores: the
 unmodified package from oracle/_ref (kind "reference"; oracle/oracle_torch.py, kind "port", only if the
 vendored copy is missing).
+
+`--dump-outputs DIR` writes a fixed, seeded sample of what the timed step returned in its last replay to
+DIR/packed.npy, DIR/scale.npy and DIR/zero_point.npy (float32, under 64 MB in all), so that two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import glob
@@ -36,6 +40,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree, which may be read-only
 
 LLAMA2_7B_LAYER = [(4096, 4096)] * 4 + [(11008, 4096)] * 2 + [(4096, 11008)]
 LLAMA3_70B_LAYER = [(8192, 8192)] * 2 + [(1024, 8192)] * 2 + [(28672, 8192)] * 2 + [(8192, 28672)]
@@ -178,9 +183,8 @@ def time_cpu_reference(mats, layers_per_step, reps, warmup):
 
 
 def time_cpu_c_port(mats, reps, warmup):
-    """C/OpenMP port of the arithmetic (oracle/quanta_oracle.c)."""
+    """C/OpenMP port of the arithmetic (oracle/quanta_oracle.c), as built by build()."""
     from oracle import oracle_c as OC
-    OC.build()
     elems = sum(m.size for m in mats)
     times = []
     for i in range(warmup + reps):
@@ -382,6 +386,36 @@ def secondary_single_gpu(device, pk, torch, Q):
     return out, launches
 
 
+DUMP_BYTES = 60_000_000                 # --dump-outputs: all files of all ranks together
+DUMP_NAMES = ("packed", "scale", "zero_point")
+
+
+def dump_outputs(out_dir, outs, rank, world, torch):
+    """Write a sample of one step's results: for each of the three arrays quantize_4bit returns, the values at
+    seeded random positions (drawn with replacement, sorted) of all matrices' arrays laid end to end in step
+    order, as float32 (packed bytes as their integer values).  The positions depend only on the array sizes,
+    so runs with the same arguments sample the same elements."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = DUMP_BYTES // 4 // len(DUMP_NAMES) // world
+    prefix = "rank%d_" % rank if world > 1 else ""
+    for k, name in enumerate(DUMP_NAMES):
+        parts = [o[k].reshape(-1) for o in outs]
+        ends = torch.tensor([p.numel() for p in parts]).cumsum(0)
+        total = int(ends[-1])
+        if total <= n:
+            idx = torch.arange(total)
+        else:
+            idx = torch.randint(0, total, (n,), generator=torch.Generator().manual_seed(1000 + k)).sort().values
+        cuts = torch.searchsorted(idx, ends).tolist()
+        vals, lo, start = [], 0, 0
+        for p, hi, end in zip(parts, cuts, ends.tolist()):
+            if hi > lo:
+                vals.append(p[(idx[lo:hi] - start).to(p.device)].float().cpu())
+            lo, start = hi, end
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), torch.cat(vals).numpy())
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
@@ -466,6 +500,8 @@ def run_ours(args, rank, world, local_rank):
     value = job_elems * BYTES_PER_ELEM / (ms * 1e-3) / 1e9
     per_gpu = total * BYTES_PER_ELEM / (ms * 1e-3) / 1e9
     launches = args.steps * (len(views) if args.per_tensor else -(-len(views) // 16))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs, rank, world, torch)
     del outs, graph
     torch.cuda.empty_cache()
 
@@ -572,7 +608,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary block (GEMM / dequantize / config 1 / TP rows)")
     ap.add_argument("--per-tensor", action="store_true", help="one quantize_4bit call (launch) per matrix instead of the batched entry")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's outputs to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
