@@ -298,7 +298,7 @@ static int dequant_multi_launch(const uint8_t* const* qs, const int64_t* numels,
         }
         for (int i = a.count; i < kDqMultiMax; ++i) { a.q[i] = nullptr; a.scale[i] = nullptr; a.zp[i] = nullptr; a.out[i] = nullptr; a.n4[i] = 0; a.chunk_base[i + 1] = a.chunk_base[a.count]; }
         const int64_t total = a.chunk_base[a.count];
-        const int64_t cap = (int64_t)kNumSMs * env_int("QUANTA_B200_DQ_MULTI_CTAS_PER_SM", 8);
+        const int64_t cap = (int64_t)kNumSMs * 8;
         cudaError_t e = launch_pdl(dequant_flat_multi_kernel<OUT, PACKED>, dim3((unsigned)(total < cap ? total : cap)), dim3(256), 0, st,
                                    a, shift_of(block), block);
         if (e != cudaSuccess) return (int)e;

@@ -24,8 +24,6 @@
 #include "common.cuh"
 
 #include <cmath>
-#include <cstdlib>
-#include <cstdio>
 
 namespace quanta {
 
@@ -205,10 +203,8 @@ struct GemmParams {
     unsigned int uq, ur;    // U / G, U % G: CTA c owns units [c uq + min(c, ur), + uq + (c < ur))
     unsigned int s_magic;   // ceil(2^32 / S) (0: S == 1): u / S without a division — a 32-bit division is ~100
     unsigned int nt_magic;  // ceil(2^32 / n_tiles) (0: n_tiles == 1)   instructions on every role's critical path
-    int my_acc;             // nacc / nmma
     int nbuf;               // accumulator buffers in TMEM (1 or 2)
     int nacc;               // independent accumulators per buffer (power of 2): consecutive MMAs rotate over them
-    int nmma;               // MMA-issuing warps (2 when nacc >= 2: tcgen05.mma dispatch is per-warp bound)
     int raw_stages, x_stages;
     int xkb;                // 64-K blocks per activation slot: 4, 2 or 1 (slot <= 32 KB)
     uint32_t raw_bytes, x_kb_bytes, x_slot_bytes, x_ring_off;
@@ -221,7 +217,6 @@ struct GemmParams {
     int ldy;                // row pitch of y in elements (N, or the full out_features of a column-parallel layer)
     int col0;               // first output column of this call inside y
     int nf4;                // 4-bit codes index the NF4 table, `scale` holds abs_max per block, zero-point unused
-    int dbg;                // experiment switches (QUANTA_B200_GEMM_DBG): 1 = no MMA, 2 = no dequant math/store
 };
 
 // Division-free index arithmetic (exactness of the multiplications is checked on the host, gemm_launch).
@@ -269,53 +264,16 @@ __device__ __forceinline__ bool elect_one() {
     return pred != 0;
 }
 
-// ---- CTA-pair helpers (CG = 2) ------------------------------------------------------------
-// Two CTAs of a cluster work on ADJACENT 128-feature tiles over the same K range and the same batch rows.  Everything
-// is private to a CTA (weight ring, dequant groups, TMEM, MMA issue, epilogue) except the activation tile, which both
-// need: each CTA loads HALF of its rows and multicasts them into both CTAs' rings, so the pair pulls every activation
-// byte out of L2 once instead of twice (at 256 batch rows the activation traffic — 128 KB per 16 KB of codes — is what
-// bounds the kernel).  A slot may be refilled when BOTH CTAs' MMAs have read it: the commit that frees it is multicast
-// too.  (The first form of the pair, one cta_group::2 MMA for both CTAs, coupled the two dequant pipelines through one
-// barrier and measured 10-25 % slower than single CTAs; it is gone.)
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r;
-}
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
-// completes `bar` in this CTA, or at the same offset in both CTAs of the pair
-template <int CG> __device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-    if (CG == 2) {
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                     ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-    } else {
-        umma_commit(bar);
-    }
-}
-// activation tile load; in a pair the rows land in both CTAs and signal both CTAs' barriers (same offsets)
-template <int CG>
-__device__ __forceinline__ void tma_load_x(uint32_t dst, const CUtensorMap* map, uint32_t bar, int32_t c0, int32_t c1, uint64_t policy) {
-    if (CG == 2) {
-        asm volatile(
-            "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster.L2::cache_hint"
-            " [%0], [%1, {%4, %5}], [%2], %3, %6;"
-            ::"r"(dst), "l"(reinterpret_cast<uint64_t>(map)), "r"(bar), "h"((uint16_t)3), "r"(c0), "r"(c1), "l"(policy)
-            : "memory");
-    } else {
-        tma_load_2d_plain(dst, map, bar, c0, c1, policy);
-    }
-}
-
 // Stream-K fix-up of one tile by `nthreads` threads (thread j): sum the fp32 partials of every
 // contributing CTA in a fixed order (deterministic), add the bias, write y.  Thread -> 4 consecutive
 // features, rows j/32, j/32 + nthreads/32, ...; kFixRows rows (float4 each) in flight per contributor.
 constexpr int kFixRows = 6;
-template <typename ACT, int CG, int NOUT>
+template <typename ACT, int NOUT>
 __device__ __noinline__ void fixup_reduce(const GemmParams& p, const GemmOutputs<NOUT>& outs, const ACT* __restrict__ bias,
-                                             const float* __restrict__ partial, int tile, int crank, int j, int nthreads) {
+                                             const float* __restrict__ partial, int tile, int j, int nthreads) {
     using AT = ActTraits<ACT>;
-    int n_idx, m_tile;
-    split_tile(tile, p, n_idx, m_tile);
-    const int n_tile = n_idx * CG + crank;
+    int n_tile, m_tile;
+    split_tile(tile, p, n_tile, m_tile);
     const int m0 = m_tile * p.mb;
     const int m_valid = min(p.mb, p.M - m0);
     const int f4 = 4 * (j & 31), mq = j >> 5, mstep = nthreads >> 5;
@@ -333,7 +291,7 @@ __device__ __noinline__ void fixup_reduce(const GemmParams& p, const GemmOutputs
         for (int i = 0; i < kFixRows; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
         for (int c = c_first; c <= c_last; ++c) {
             const int wc = (tile == tile_of_unit(first_unit((unsigned int)c, p), p)) ? 0 : 1;
-            const float* src = partial + (((size_t)c * 2 + wc) * CG + crank) * slot_elems + f4;
+            const float* src = partial + ((size_t)c * 2 + wc) * slot_elems + f4;
             float4 v[kFixRows];
 #pragma unroll
             for (int i = 0; i < kFixRows; ++i) {
@@ -366,7 +324,7 @@ __device__ __noinline__ void fixup_reduce(const GemmParams& p, const GemmOutputs
     }
 }
 
-template <typename ACT, int BITS, int CG, int NOUT>
+template <typename ACT, int BITS, int NOUT>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_x,
                   const __grid_constant__ CUtensorMap tmap_s, const __grid_constant__ CUtensorMap tmap_z,
@@ -382,25 +340,11 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
     __shared__ int fin_tile;            // tile whose stream-K fix-up is done by the whole CTA at the end (-1: none)
     __shared__ __align__(1024) float stage[16][kTileN];        // epilogue transpose buffer (8 KB)
     __shared__ uint32_t nf4_pairs[256];                        // NF4: byte -> (level[lo nibble], level[hi nibble]) in the act type
-#ifdef QUANTA_GEMM_TRACE
-    __shared__ long long trace[8][48];
-    const bool tr = (p.dbg & 8) && blockIdx.x == 0;
-    int tri = 0;
-    const long long t_start = clock64();
-#define TRACE2(role, cond) do { if (tr && (cond) && tri < 48) trace[role][tri++] = clock64() - t_start; } while (0)
-#define TRACE(role) do { if (tr && tri < 48) trace[role][tri++] = clock64() - t_start; } while (0)
-#else
-#define TRACE2(role, cond) do { } while (0)
-#define TRACE(role) do { } while (0)
-#endif
 
     const uint32_t smem = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const int tid = threadIdx.x, lane = tid & 31;
     const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);       // warp-uniform for the compiler
-    // CG = 2: the two CTAs of a cluster form a pair: they walk the same unit range on adjacent 128-feature tiles
-    // and share the activation loads (see the pair helpers above).  `cta` is the scheduling unit (CTA or pair).
-    const uint32_t crank = CG == 2 ? cluster_ctarank() : 0u;
-    const unsigned int cta = blockIdx.x / CG;
+    const unsigned int cta = blockIdx.x;
 
     // shared memory: [raw ring: raw_stages x 16|32 KB][x ring: x_stages x (xkb x mb x 128 B)]
     auto r_addr = [&](int s) { return smem + (uint32_t)s * p.raw_bytes; };
@@ -434,15 +378,14 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
             if (p.vec4) { prefetch_tensormap(&tmap_s); prefetch_tensormap(&tmap_z); }
         }
         __syncwarp();
-        if (CG == 2) cluster_arrive();                       // checked in; the matching wait comes after the stream
-        else asm volatile("barrier.arrive 2, %0;" ::"n"(kGemmThreads) : "memory");
+        asm volatile("barrier.arrive 2, %0;" ::"n"(kGemmThreads) : "memory");
         const uint64_t pol_w = policy_evict_first();         // weights are streamed once
         int slot = 0, issued = 0;
         uint32_t ph = 0;
         while (walk.next(tile, s0, s1)) {
             int n_idx, m_idx;
             split_tile(tile, p, n_idx, m_idx);
-            const int n0 = (n_idx * CG + (int)crank) * kTileN;
+            const int n0 = n_idx * kTileN;
             for (int s = s0; s < s1; ++s) {
                 if (issued >= p.raw_stages) mbar_wait(&raw_empty[slot], ph ^ 1);
                 if (elect_one()) {
@@ -459,24 +402,21 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                         tma_load_2d_plain(r_addr(slot) + kRawCodeBytes, &tmap_s, bar, s * kKbPerStage, n0, pol_w);
                         tma_load_2d_plain(r_addr(slot) + kRawCodeBytes + 2048u, &tmap_z, bar, s * kKbPerStage, n0, pol_w);
                     }
-                    TRACE(0);
                 }
                 __syncwarp();
                 ++issued;
                 if (++slot == p.raw_stages) { slot = 0; ph ^= 1; }
             }
         }
-        if (CG == 2) cluster_wait();
     } else if (warp == 1) {
         // ===== activation tiles: xkb 64-K blocks per slot =====
         if (lane == 0) {
-            for (int s = 0; s < p.x_stages; ++s) { mbar_init(&x_full[s], 1); mbar_init(&x_empty[s], CG); }   // freed by both CTAs' MMAs
+            for (int s = 0; s < p.x_stages; ++s) { mbar_init(&x_full[s], 1); mbar_init(&x_empty[s], 1); }
             fence_barrier_init();
             prefetch_tensormap(&tmap_x);
         }
         __syncwarp();
-        if (CG == 2) { cluster_arrive(); cluster_wait(); }   // the peer's barriers must exist before the first load
-        else asm volatile("barrier.arrive 2, %0;" ::"n"(kGemmThreads) : "memory");
+        asm volatile("barrier.arrive 2, %0;" ::"n"(kGemmThreads) : "memory");
         const uint64_t pol_x = policy_evict_last();          // activations are re-read by every CTA
         asm volatile("griddepcontrol.wait;" ::: "memory");   // x may be the previous kernel's output
         int slot = 0, issued = 0;
@@ -484,20 +424,18 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         while (walk.next(tile, s0, s1)) {
             int n_idx, m_idx;
             split_tile(tile, p, n_idx, m_idx);
-            const int m0 = m_idx * p.mb + (int)crank * (p.mb / CG);                  // this CTA loads (and multicasts) its half of the rows
-            const uint32_t half_off = crank * (uint32_t)(p.mb / CG) * 128u;          // where they go inside a 64-K block of the slot
+            const int m0 = m_idx * p.mb;
             for (int s = s0; s < s1; ++s) {
                 for (int j = 0; j < kKbPerStage; j += p.xkb) {
                     if (issued >= p.x_stages) mbar_wait(&x_empty[slot], ph ^ 1);
                     if (elect_one()) {
-                        mbar_arrive_expect_tx(&x_full[slot], p.x_slot_bytes);               // all rows: own loads + the peer's
+                        mbar_arrive_expect_tx(&x_full[slot], p.x_slot_bytes);
                         // blocks past the end of K are out of bounds and arrive zero-filled
                         for (int jj = 0; jj < p.xkb; ++jj)
-                            tma_load_x<CG>(x_addr(slot) + (uint32_t)jj * p.x_kb_bytes + half_off, &tmap_x, smem_u32(&x_full[slot]),
-                                           (s * kKbPerStage + j + jj) * kBlockK, m0, pol_x);
+                            tma_load_2d_plain(x_addr(slot) + (uint32_t)jj * p.x_kb_bytes, &tmap_x, smem_u32(&x_full[slot]),
+                                              (s * kKbPerStage + j + jj) * kBlockK, m0, pol_x);
                     }
                     __syncwarp();
-                    TRACE2(3, lane == 0);
                     ++issued;
                     if (++slot == p.x_stages) { slot = 0; ph ^= 1; }
                 }
@@ -508,75 +446,65 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
             tmem_alloc(smem_u32(&tmem_base_slot), kTmemCols);
         } else if (warp == 3 && lane == 0) {
             for (int s = 0; s < kDqGroups; ++s) { mbar_init(&a_full[s], kDqGroupWarps); mbar_init(&a_empty[s], 1); }
-            for (int s = 0; s < 2; ++s) { mbar_init(&d_full[s], p.nmma); mbar_init(&d_empty[s], kEpiWarps); }
+            for (int s = 0; s < 2; ++s) { mbar_init(&d_full[s], 1); mbar_init(&d_empty[s], kEpiWarps); }
             fence_barrier_init();
         }
         __syncwarp();
         tc_fence_before();
-        if (CG == 2) { cluster_arrive(); cluster_wait(); }
-        else asm volatile("barrier.sync 2, %0;" ::"n"(kGemmThreads) : "memory");
+        asm volatile("barrier.sync 2, %0;" ::"n"(kGemmThreads) : "memory");
     }
     tc_fence_after();
     const uint32_t tmem = tmem_base_slot;
 
-    if (warp == 2 || (warp == 3 && p.nmma == 2)) {
-        // ===== MMA issuers: the whole warp walks the schedule, one elected lane issues =====
-        // A tcgen05.mma costs ~70 cycles of dispatch whatever its size (the tensor pipe itself needs only
-        // N/2 cycles), so a stage is >= 1120 cycles of issue plus ~600 cycles of barrier waits and
-        // commits.  With two issuers (small batches) warp 2 takes the even stages and warp 3 the odd
-        // ones — one dequant group each — so one warp's waits hide behind the other's issue; each
-        // warp rotates over its own half of the accumulators (the epilogue adds all of them up).
-        const int mw = warp - 2;
+    if (warp == 2) {
+        // ===== MMA issuer: the whole warp walks the schedule, one elected lane issues =====
+        // (one issuer is enough: the body is bound by the dequant groups, not by the ~70 cycles of
+        // dispatch per tcgen05.mma; DESIGN §4.1)
         const uint32_t idesc = (1u << 4) | (AT::kFmt << 7) | (AT::kFmt << 10) |
                                ((uint32_t)(p.mb >> 3) << 17) | ((uint32_t)(kTileN >> 4) << 24);
         const uint32_t kb_desc = p.x_kb_bytes >> 4;          // descriptor step between 64-K blocks of one slot
-        const uint32_t my_acc = (uint32_t)p.my_acc;                   // accumulators of this warp (power of 2)
+        const uint32_t nacc = (uint32_t)p.nacc;
         int sx = 0, seg = 0, sc = 0;
         uint32_t px = 0;
         while (walk.next(tile, s0, s1)) {
             const int buf = p.nbuf == 2 ? (seg & 1) : 0;
             const uint32_t use = (uint32_t)(p.nbuf == 2 ? (seg >> 1) : seg);      // how often `buf` was used before
             mbar_wait(&d_empty[buf], (use & 1) ^ 1);   // the epilogues have drained this accumulator
-            const uint32_t tmem_d = tmem + kDBase + (uint32_t)((buf * p.nacc + mw * (int)my_acc) * p.mb);
-            uint32_t touched = 0;                            // own accumulators already written in this segment
+            const uint32_t tmem_d = tmem + kDBase + (uint32_t)(buf * p.nacc * p.mb);
+            uint32_t touched = 0;                            // accumulators already written in this segment
             for (int s = s0; s < s1; ++s, ++sc) {
                 const int nkb = min(kKbPerStage, p.total_kb - s * kKbPerStage);
                 const int g = sc & 1;                        // dequant group = A buffer
-                if (p.nmma == 1 || g == mw) mbar_wait(&a_full[g], (uint32_t)(sc >> 1) & 1u);   // the stage's 4 A tiles are in TMEM
+                mbar_wait(&a_full[g], (uint32_t)(sc >> 1) & 1u);   // the stage's 4 A tiles are in TMEM
                 const uint32_t ta = tmem + (uint32_t)(g * kKbPerStage * kACols);
-                TRACE2(2, lane == 0);
 #pragma unroll
                 for (int j = 0; j < kKbPerStage; ++j) {
                     const int jj = j & (p.xkb - 1);
-                    const bool mine = p.nmma == 1 || (sc & 1) == mw;
-                    if (mine) {
-                        if (jj == 0) mbar_wait(&x_full[sx], px);       // activation slot landed
-                        tc_fence_after();
-                        const bool live = j < nkb && !(p.dbg & 1);
-                        uint32_t acc_idx[4], acc_flag[4];    // computed by every lane: stays warp-uniform
+                    if (jj == 0) mbar_wait(&x_full[sx], px);       // activation slot landed
+                    tc_fence_after();
+                    const bool live = j < nkb;
+                    uint32_t acc_idx[4], acc_flag[4];    // computed by every lane: stays warp-uniform
 #pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            acc_idx[k] = (uint32_t)(4 * j + k) & (my_acc - 1u);
-                            acc_flag[k] = (touched >> acc_idx[k]) & 1u;
-                            if (live) touched |= 1u << acc_idx[k];
-                        }
-                        if (elect_one()) {
-                            if (live) {
-                                const uint64_t db = smem_desc_sw128(x_addr(sx)) + (uint64_t)(jj * kb_desc);
-#pragma unroll
-                                for (int k = 0; k < kBlockK / 16; ++k)    // K = 16 per MMA: 8 TMEM columns of A, 32 bytes of B
-                                    umma_f16_ts(tmem_d + acc_idx[k] * (uint32_t)p.mb, ta + (uint32_t)(j * kACols + 8 * k),
-                                                db + 2 * k, idesc, acc_flag[k]);
-                            }
-                            // both arrive when the MMAs above have read their operands
-                            if (jj == p.xkb - 1) umma_commit_pair<CG>(&x_empty[sx]);   // in a pair: frees the slot in both CTAs
-                            if (j == kKbPerStage - 1) umma_commit(&a_empty[g]);
-                        }
-                        __syncwarp();
+                    for (int k = 0; k < 4; ++k) {
+                        acc_idx[k] = (uint32_t)(4 * j + k) & (nacc - 1u);
+                        acc_flag[k] = (touched >> acc_idx[k]) & 1u;
+                        if (live) touched |= 1u << acc_idx[k];
                     }
+                    if (elect_one()) {
+                        if (live) {
+                            const uint64_t db = smem_desc_sw128(x_addr(sx)) + (uint64_t)(jj * kb_desc);
+#pragma unroll
+                            for (int k = 0; k < kBlockK / 16; ++k)    // K = 16 per MMA: 8 TMEM columns of A, 32 bytes of B
+                                umma_f16_ts(tmem_d + acc_idx[k] * (uint32_t)p.mb, ta + (uint32_t)(j * kACols + 8 * k),
+                                            db + 2 * k, idesc, acc_flag[k]);
+                        }
+                        // both arrive when the MMAs above have read their operands
+                        if (jj == p.xkb - 1) umma_commit(&x_empty[sx]);
+                        if (j == kKbPerStage - 1) umma_commit(&a_empty[g]);
+                    }
+                    __syncwarp();
                     if (jj == p.xkb - 1) { if (++sx == p.x_stages) { sx = 0; px ^= 1; } }
                 }
-                TRACE2(2, lane == 0);
             }
             if (elect_one()) umma_commit(&d_full[buf]);
             __syncwarp();
@@ -589,13 +517,12 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         const int row = 32 * quarter + lane;
         const int etid = tid - 32 * kFirstEpiWarp;
         if (etid == 0 && p.y_tma) { for (int o = 0; o < (NOUT == 1 ? 1 : p.n_out); ++o) prefetch_tensormap(&outs.maps[o]); }
-        int seg = 0, esc = 0;                 // esc: CTA-wide stage counter at the start of the segment
+        int seg = 0;
         while (walk.next(tile, s0, s1)) {
             const int buf = p.nbuf == 2 ? (seg & 1) : 0;
             const uint32_t use = (uint32_t)(p.nbuf == 2 ? (seg >> 1) : seg);
-            int n_idx, m_tile;
-            split_tile(tile, p, n_idx, m_tile);
-            const int n_tile = n_idx * CG + (int)crank;
+            int n_tile, m_tile;
+            split_tile(tile, p, n_tile, m_tile);
             const int gn = n_tile * kTileN + row, m0 = m_tile * p.mb;
             const bool n_ok = gn < p.N;
             const int m_valid = min(p.mb, p.M - m0);
@@ -604,12 +531,10 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
             const float b = (bias != nullptr && n_ok) ? AT::to_float(bias[gn]) : 0.0f;
             // this CTA's partial slot for the tile: 0 if the tile is the first one the CTA touches, else 1
             const int which = (tile == tile_of_unit(first_unit(cta, p), p)) ? 0 : 1;
-            float* mine = partial + (((size_t)cta * 2 + which) * CG + crank) * (size_t)(kTileN * p.mb);
+            float* mine = partial + ((size_t)cta * 2 + which) * (size_t)(kTileN * p.mb);
 
-            TRACE2(4, etid == 0);
             mbar_wait(&d_full[buf], use & 1);
             tc_fence_after();
-            TRACE2(4, etid == 0);
             const uint32_t taddr = tmem + ((uint32_t)(32 * quarter) << 16) + kDBase + (uint32_t)(buf * p.nacc * p.mb);
             // store mapping: thread -> 4 consecutive features (f4..f4+3), batch rows etid/32 + 4q
             const int f4 = 4 * (etid & 31);
@@ -618,30 +543,19 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
 #pragma unroll
             for (int e = 0; e < 4; ++e) b4[e] = (bias != nullptr && gn4 + e < p.N) ? AT::to_float(bias[gn4 + e]) : 0.0f;
             const bool vec_ok = p.vec_store && gn4 + 3 < p.N;
-            // accumulators the MMA warps wrote in this segment: each warp issues 4 MMAs per 64-K block of
-            // its half of the stage (all of it with one issuer), rotating over its own my_acc accumulators
-            const int my_acc = p.my_acc;
+            // accumulators the MMA warp wrote in this segment: 4 MMAs per 64-K block, rotating over nacc
             const int last_nkb = (s1 == p.S) ? p.total_kb - (p.S - 1) * kKbPerStage : kKbPerStage;
-            int kb_w[2];
-            if (p.nmma == 1) { kb_w[0] = (s1 - s0 - 1) * kKbPerStage + last_nkb; kb_w[1] = 0; }
-            else {
-                // warp w issued the stages whose CTA-wide stage counter has parity w
-                kb_w[0] = kb_w[1] = 0;
-                for (int s = s0; s < s1; ++s) kb_w[(esc + (s - s0)) & 1] += (s == p.S - 1) ? last_nkb : kKbPerStage;
-            }
+            const int nv = min(p.nacc, 4 * ((s1 - s0 - 1) * kKbPerStage + last_nkb));
             for (int c0 = 0; c0 < p.mb; c0 += 16) {
                 uint32_t r[16];
 #pragma unroll
                 for (int j = 0; j < 16; ++j) r[j] = 0u;
-                for (int w = 0; w < p.nmma; ++w) {
-                    const int nv = min(my_acc, 4 * kb_w[w]);
-                    for (int a = 0; a < nv; ++a) {
-                        uint32_t t[16];
-                        tmem_ld16(taddr + (uint32_t)((w * my_acc + a) * p.mb) + c0, t);
-                        tmem_ld_wait();
+                for (int a = 0; a < nv; ++a) {
+                    uint32_t t[16];
+                    tmem_ld16(taddr + (uint32_t)(a * p.mb) + c0, t);
+                    tmem_ld_wait();
 #pragma unroll
-                        for (int j = 0; j < 16; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(t[j]));
-                    }
+                    for (int j = 0; j < 16; ++j) r[j] = __float_as_uint(__uint_as_float(r[j]) + __uint_as_float(t[j]));
                 }
                 if (whole && p.y_tma) {
                     // Whole tile: bias, 16-bit conversion, [16 rows x 128 features] staged in shared memory
@@ -700,7 +614,6 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                 }
             }
             if (whole && p.y_tma && etid == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging free for the next segment
-            TRACE2(4, etid == 0);
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&d_empty[buf]);   // accumulator may be overwritten
@@ -713,10 +626,10 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                 asm volatile("bar.sync 1, %0;" ::"n"(32 * kEpiWarps) : "memory");
                 if (etid == 0) {
                     __threadfence();
-                    const unsigned int old = atomicAdd(&counters[tile * CG + (int)crank], 1u);
+                    const unsigned int old = atomicAdd(&counters[tile], 1u);
                     __threadfence();
                     const int last = (old == (unsigned int)(c_last - c_first)) ? 1 : 0;
-                    if (last) counters[tile * CG + (int)crank] = 0u;      // leave the workspace clean for the next call
+                    if (last) counters[tile] = 0u;      // leave the workspace clean for the next call
                     fix_flag = last;
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(32 * kEpiWarps) : "memory");
@@ -726,12 +639,11 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                         // warps (5x the loads in flight) after the role loops
                         if (etid == 0) fin_tile = tile;
                     } else {
-                        fixup_reduce<ACT, CG, NOUT>(p, outs, bias, partial, tile, (int)crank, etid, 32 * kEpiWarps);
+                        fixup_reduce<ACT, NOUT>(p, outs, bias, partial, tile, etid, 32 * kEpiWarps);
                     }
                 }
                 asm volatile("bar.sync 1, %0;" ::"n"(32 * kEpiWarps) : "memory");      // fix_flag is reused
             }
-            esc += s1 - s0;
             ++seg;
         }
     } else if (warp >= kFirstDqWarp) {
@@ -754,7 +666,7 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         auto fetch_params = [&](int t, int s) {
             int n_idx, m_idx;
             split_tile(t, p, n_idx, m_idx);
-            const int gn = (n_idx * CG + (int)crank) * kTileN + row;
+            const int gn = n_idx * kTileN + row;
             const int64_t rbase = (int64_t)(gn < p.N ? gn : p.N - 1) * p.scale_stride;
             const int kb = s * kKbPerStage;
 #pragma unroll
@@ -791,9 +703,7 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                         skip(kDqGroups);
                         if (a_ok) fetch_params(a_tile, a_s); // lands while this stage is processed
                     }
-                    TRACE2(1, lane == 0 && quarter == 0 && half == 0 && group == 0 && sc >= 4 && sc <= 8);
                     mbar_wait(&raw_full[rslot], rph);
-                    TRACE2(1, lane == 0 && quarter == 0 && half == 0 && group == 0 && sc >= 4 && sc <= 8);
 
                     const uint32_t rrow = r_addr(rslot) + (uint32_t)row * 128u;
                     const uint32_t sw = (uint32_t)(row & 7);
@@ -806,10 +716,9 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                     // the MMAs that read this group's A buffer two stages ago are done
                     mbar_wait(&a_empty[group], ((uint32_t)(sc >> 1) & 1u) ^ 1u);
                     tc_fence_after();
-                    TRACE2(1, lane == 0 && quarter == 0 && half == 0 && group == 0 && sc >= 4 && sc <= 8);
 #pragma unroll
                     for (int j = 0; j < kKbPerStage; ++j) {
-                        if (j < nkb && !(p.dbg & 2)) {
+                        if (j < nkb) {
                             uint32_t out[16];
                             if (BITS == 4 && p.nf4) {
                                 // NF4: one shared-memory lookup per code byte gives the K-adjacent pair
@@ -848,10 +757,8 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                             }
                             tmem_st16(a_addr + (uint32_t)(j * kACols), out);
                         }
-                        TRACE2(1, lane == 0 && quarter == 0 && half == 0 && group == 0 && sc >= 4 && sc <= 8);
-                    }
+                        }
                     tmem_st_wait();
-                    TRACE2(1, lane == 0 && quarter == 0 && half == 0 && group == 0 && sc >= 4 && sc <= 8);
                     tc_fence_before();
                     __syncwarp();
                     if (lane == 0) {
@@ -872,25 +779,18 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         asm volatile("bar.sync 3, %0;" ::"n"(32 * (kEpiWarps + kDqWarps)) : "memory");
         const int ft = *reinterpret_cast<volatile int*>(&fin_tile);
         if (ft >= 0)
-            fixup_reduce<ACT, CG, NOUT>(p, outs, bias, partial, ft, (int)crank, tid - 32 * kFirstEpiWarp, 32 * (kEpiWarps + kDqWarps));
+            fixup_reduce<ACT, NOUT>(p, outs, bias, partial, ft, tid - 32 * kFirstEpiWarp, 32 * (kEpiWarps + kDqWarps));
     }
     if (tid == 32 * kFirstEpiWarp) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");       // y stores have landed
     tc_fence_before();
     __syncthreads();
-    if (CG == 2) { cluster_arrive(); cluster_wait(); }       // the peer may still be signalling into this CTA
     if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem, kTmemCols); }
-#ifdef QUANTA_GEMM_TRACE
-    if (tr && tid == 0) {
-        printf("end %lld\n", clock64() - t_start);
-        for (int r = 0; r < 8; ++r) { printf("role %d:", r); for (int i = 0; i < 48; ++i) printf(" %lld", trace[r][i]); printf("\n"); }
-    }
-#endif
 }
 
 // ---- host side --------------------------------------------------------------
 
 
-// Number of scheduling units (CTAs, or CTA pairs when cg = 2): every SM with equal contiguous unit
+// Number of CTAs: every SM with equal contiguous unit
 // ranges (stream-K), or tiles x s units whose ranges coincide with tile boundaries (s = 1: no
 // partials at all).  Costs in SM cycles, from the measurements in DESIGN.md: a stage (256 K) costs
 // the MMA warp ~600 cycles of barrier traffic plus 16 MMAs of max(70, mb/2) cycles each, the
@@ -898,11 +798,11 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
 // tiles (re-read by every tile) out of L2 at ~29 B/cycle; a partial costs its fp32 store, ~4000
 // cycles of release/acquire latency and the last arriver's (latency-bound) reads of every
 // contributor's tile.
-static int choose_units(int tiles, int S, int mb, int raw_bytes, int cg) {
-    const int max_units = kNumSMs / cg;
+static int choose_units(int tiles, int S, int mb, int raw_bytes) {
+    const int max_units = kNumSMs;
     const long long U = (long long)tiles * S;
     const double mma = 600.0 + 16.0 * (mb / 2.0 > 70.0 ? mb / 2.0 : 70.0);
-    const double pull = (512.0 * mb / cg + raw_bytes) / 29.0;
+    const double pull = (512.0 * mb + raw_bytes) / 29.0;
     const double stage = fmax(fmax(mma, 930.0), pull);
     const double tile_io = (double)kTileN * mb * 4.0 / 32.0;
     int best = 1;
@@ -933,17 +833,16 @@ size_t gemm_workspace_bytes(int64_t M, int64_t) {
     return (size_t)kCounterBytes + (size_t)kNumSMs * 2 * kTileN * (size_t)mb * sizeof(float) + 512;
 }
 
-template <typename ACT, int BITS, int CG, int NOUT>
-static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const float* scale, const float* zp,
+template <typename ACT, int BITS, int NOUT>
+static int gemm_tc_launch(GemmParams& p, const ACT* x, const uint8_t* wq, const float* scale, const float* zp,
                           const ACT* bias, void* const* ys, int64_t M, int64_t N, int64_t K, void* workspace, size_t ws_bytes,
                           cudaStream_t st) {
     const int mb = p.mb;
-    const int tiles = p.n_tiles * p.m_tiles;               // scheduling tiles: CG adjacent 128-feature tiles each
-    if (tiles * CG > kMaxTiles) return QUANTA_EUNSUPPORTED;
+    const int tiles = p.n_tiles * p.m_tiles;
+    if (tiles > kMaxTiles) return QUANTA_EUNSUPPORTED;
     if ((unsigned long long)tiles * (unsigned long long)p.S * (unsigned long long)(kNumSMs + 1) >= (1ull << 32)) return QUANTA_EUNSUPPORTED;
     p.U = (unsigned int)tiles * (unsigned int)p.S;
-    p.G = choose_units(tiles, p.S, mb, BITS == 4 ? 16384 : 32768, CG);
-    { const int v = env_int("QUANTA_B200_GEMM_CTAS", 0); if (v >= 1 && v <= kNumSMs / CG && (unsigned int)v <= p.U) p.G = v; }
+    p.G = choose_units(tiles, p.S, mb, BITS == 4 ? 16384 : 32768);
     p.uq = p.U / (unsigned int)p.G;
     p.ur = p.U % (unsigned int)p.G;
     {
@@ -957,8 +856,7 @@ static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const 
         if (!magic_for((unsigned int)p.S, p.U, &p.s_magic) || !magic_for((unsigned int)p.n_tiles, (unsigned long long)tiles, &p.nt_magic))
             return QUANTA_EUNSUPPORTED;
     }
-    p.my_acc = p.nacc / p.nmma;
-    p.x_kb_bytes = (uint32_t)mb * 128u;                     // one 64-K block of the activation tile (all rows: a pair multicasts)
+    p.x_kb_bytes = (uint32_t)mb * 128u;                     // one 64-K block of the activation tile
     p.xkb = p.x_kb_bytes <= 8192u ? 4 : (p.x_kb_bytes <= 16384u ? 2 : 1);    // activation slots of at most 32 KB
     p.x_slot_bytes = p.x_kb_bytes * (uint32_t)p.xkb;
     p.raw_bytes = (BITS == 4 ? 16384u : 32768u) + (p.vec4 ? 4096u : 0u);    // codes (+ scale / zero-point tiles)
@@ -974,7 +872,7 @@ static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const 
     p.x_stages = x_stages;
     p.x_ring_off = (uint32_t)raw_stages * p.raw_bytes;
 
-    const size_t need = (size_t)kCounterBytes + (size_t)p.G * CG * 2 * kTileN * (size_t)mb * sizeof(float) + 256;
+    const size_t need = (size_t)kCounterBytes + (size_t)p.G * 2 * kTileN * (size_t)mb * sizeof(float) + 256;
     if (!workspace || ws_bytes < need) return QUANTA_EWORKSPACE;
     uint8_t* ws = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~uintptr_t(255));
     unsigned int* counters = reinterpret_cast<unsigned int*>(ws);
@@ -986,7 +884,7 @@ static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const 
                                 128, kTileN, CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
     rc = make_tensor_map_2d(&tmap_x, ActTraits<ACT>::kTma, 2, x, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, kBlockK,
-                            (uint32_t)(mb / CG), CU_TENSOR_MAP_SWIZZLE_128B);
+                            (uint32_t)mb, CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
 
     CUtensorMap tmap_s = tmap_w, tmap_z = tmap_w;          // placeholders unless the parameters ride on TMA
@@ -1010,7 +908,6 @@ static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const 
     }
     p.vec_store = (aligned8 && (p.ldy & 3) == 0 && (p.col0 & 3) == 0) ? 1 : 0;
     p.y_tma = (aligned16 && (p.ldy & 7) == 0) ? 1 : 0;
-    if (env_int("QUANTA_B200_GEMM_YTMA", 1) == 0) p.y_tma = 0;
     if (p.y_tma) {
         // window [M, col0 + N] of each buffer: features past this call's columns are clipped by the map
         for (int o = 0; o < p.n_out; ++o) {
@@ -1019,28 +916,19 @@ static int gemm_launch_cg(GemmParams& p, const ACT* x, const uint8_t* wq, const 
             if (rc) return rc;
         }
     }
-    auto kern = gemm_wna16_kernel<ACT, BITS, CG, NOUT>;
+    auto kern = gemm_wna16_kernel<ACT, BITS, NOUT>;
     const int smem = (int)(p.x_ring_off + (uint32_t)p.x_stages * p.x_slot_bytes + 1024);
     if (int e = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return e;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(p.G * CG));
+    cfg.gridDim = dim3((unsigned)p.G);
     cfg.blockDim = dim3(kGemmThreads);
     cfg.dynamicSmemBytes = (size_t)smem;
     cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    int na = 0;
-    if (env_int("QUANTA_B200_GEMM_PDL", 1)) {
-        attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[na].val.programmaticStreamSerializationAllowed = 1;
-        ++na;
-    }
-    if (CG == 2) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = CG; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = na;
+    cfg.numAttrs = 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmap_w, tmap_x, tmap_s, tmap_z, outs, scale, zp, bias, counters, partial, p);
     return cuda_status(e != cudaSuccess ? e : cudaGetLastError());
 }
@@ -1065,42 +953,25 @@ static int gemm_launch(const ACT* x, const uint8_t* wq, const float* scale, cons
     if (sync) return QUANTA_EUNSUPPORTED;                    // the in-kernel completion exists in the small-batch kernel only
     GemmParams p;
     p.M = (int)M; p.N = (int)N; p.K = (int)K;
-    const int n_tiles = (int)((N + kTileN - 1) / kTileN);
-    // CTA pairs (CG = 2: adjacent feature tiles, the activation tile loaded once and multicast to both CTAs) halve the
-    // L2 reads of the activations — and measured no faster (M = 256: 42.8 vs 42.1 us on 4096 x 14336, 32.1 vs 31.8 on
-    // 14336 x 4096; M = 64 / 128 1-4 % slower): every SM still has to take in the whole 128 KB tile per 256-K stage
-    // (41 B/cycle at the measured stage time), so the bound is the SM's inbound path, not L2.  Off unless
-    // QUANTA_B200_GEMM_PAIR=1 (kept working by tests/test_gpu_gemm.py::test_cta_pair_multicast_mode).
-    int cg = 1;
-    if (env_int("QUANTA_B200_GEMM_PAIR", 0) == 1 && n_tiles >= 2 && n_out == 1) cg = 2;
-    const int mb_step = 16 * cg;                             // each CTA of a pair holds mb / 2 rows, a multiple of 16
-    int mb = (int)((M + mb_step - 1) / mb_step * mb_step);
+    int mb = (int)((M + 15) / 16 * 16);
     if (mb > 256) mb = 256;
-    { const int cap = env_int("QUANTA_B200_GEMM_MB", 0); if (cap >= 16 && cap % 16 == 0 && mb > cap) mb = cap; }
     p.mb = mb;
     p.m_tiles = (int)((M + mb - 1) / mb);
-    p.n_tiles = (n_tiles + cg - 1) / cg;
+    p.n_tiles = (int)((N + kTileN - 1) / kTileN);
     p.total_kb = (int)(K / kBlockK);
     p.S = (p.total_kb + kKbPerStage - 1) / kKbPerStage;
     // accumulators: nbuf x nacc x mb <= 256 TMEM columns
     p.nacc = mb <= 16 ? 8 : (mb <= 64 ? 4 : (mb <= 128 ? 2 : 1));
     p.nbuf = (2 * p.nacc * mb <= kTmemCols - kDBase) ? 2 : 1;
-    // a second MMA-issuing warp (even / odd stages) is implemented but measured no faster: the body is
-    // bound by the dequant groups, not by the issuer (QUANTA_B200_GEMM_NMMA=2 enables it)
-    p.nmma = 1;
-    if (env_int("QUANTA_B200_GEMM_NMMA", 1) == 2 && p.nacc >= 2) p.nmma = 2;
-    p.dbg = 0;
     p.nf4 = nf4;
     p.n_out = n_out; p.ldy = (int)ldy; p.col0 = (int)col0;
-    p.dbg = env_int("QUANTA_B200_GEMM_DBG", 0);
     p.scale_stride = (int)(K / block);
     int bs = 0; while ((int64_t)(kBlockK << bs) < block) ++bs;
     p.block_shift = bs;
     p.vec4 = (bs == 0 && (p.scale_stride & 3) == 0 &&
               ((reinterpret_cast<uintptr_t>(scale) | reinterpret_cast<uintptr_t>(zp)) & 15) == 0) ? 1 : 0;
-    if (n_out > 1) return gemm_launch_cg<ACT, BITS, 1, kMaxOut>(p, x, wq, scale, zp, bias, ys, M, N, K, workspace, ws_bytes, st);
-    if (cg == 2) return gemm_launch_cg<ACT, BITS, 2, 1>(p, x, wq, scale, zp, bias, ys, M, N, K, workspace, ws_bytes, st);
-    return gemm_launch_cg<ACT, BITS, 1, 1>(p, x, wq, scale, zp, bias, ys, M, N, K, workspace, ws_bytes, st);
+    if (n_out > 1) return gemm_tc_launch<ACT, BITS, kMaxOut>(p, x, wq, scale, zp, bias, ys, M, N, K, workspace, ws_bytes, st);
+    return gemm_tc_launch<ACT, BITS, 1>(p, x, wq, scale, zp, bias, ys, M, N, K, workspace, ws_bytes, st);
 }
 
 }  // namespace quanta

@@ -42,8 +42,6 @@
 // the 1e-2 tolerance of rows G1/G2.
 #include "common.cuh"
 
-#include <cstdio>
-#include <cstdlib>
 #include <type_traits>
 
 namespace quanta {
@@ -58,7 +56,8 @@ constexpr int sm_threads(int xw) { return kSmConsThreads + 64 + 32 * xw; }   // 
 constexpr int kSmKGran = 256;              // K must be a multiple of this (16-byte scale rows; a partial last step is zero-filled)
 constexpr int kSmMaxRing = 8;
 constexpr int kSmMaxXRing = 4;             // activation slots (one stage each)
-constexpr int kSmStartWindow = 2;          // default number of stages requested before the first one has landed
+constexpr int kSmStartWindow = 2;          // stages requested before the first one has landed
+constexpr int kSmMaxM = 16;                // batch rows served (NB = 2 column blocks of 8)
 constexpr int kSmMaxOut = 8;
 constexpr int kSmCounterBytes = 64 * 1024; // same workspace header as gemm.cu (zero before, zero after)
 
@@ -82,13 +81,6 @@ __constant__ float kSmNf4Levels[16] = {
     0.24611230194568634f, 0.33791524171829224f, 0.44070982933044434f, 0.5626170039176941f,
     0.7229568362236023f, 1.0f};
 
-// The experiment switches cost ~25 instructions per unit in the consumers' loop: compiled in only on request.
-#ifdef QUANTA_SMALL_DBG
-#define SM_DBG(p, bit) (((p).dbg & (bit)) != 0)
-#else
-#define SM_DBG(p, bit) false
-#endif
-
 // Timeline of one launch (-DQUANTA_SMALL_TRACE build only): per CTA 40 clock64 stamps relative to kernel entry, + globaltimer at
 // entry / exit in slots 38 / 39.  Read back with quanta_debug_small_trace().
 #ifdef QUANTA_SMALL_TRACE
@@ -109,11 +101,9 @@ struct SmallParams {
     int m_pad;              // 8 * NB
     int R;                  // weight ring stages
     int XR;                 // activation ring slots (<= kSmMaxXRing)
-    int window;             // stages requested before the first one has landed
+    int window;             // stages requested before the first one has landed (kSmStartWindow, at most R)
     int ldy, col0, n_out;
     int vec_y;              // 8-byte y stores are aligned in every output buffer
-    int dbg;                // experiment switches (QUANTA_B200_SMALL_DBG; only in a -DQUANTA_SMALL_DBG build): 1 no compute,
-                            // 2 no x staging, 4 no epilogue, 8 no TMA
     uint32_t x_off;         // x ring
     uint32_t x_slot_bytes;  // NB * kBlk * (1024 fragment bytes + 32 block-sum bytes)
     uint32_t lut_off;       // NF4 pair table (kSmLutBytes), unused otherwise
@@ -416,7 +406,6 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
             uint32_t ph = 0;
             while (walk.next(tile, s0, s1, final_seg)) {
                 for (int step = s0; step < s1; ++step, ++i) {
-                    if (SM_DBG(p, 8)) break;
                     if (i == 0) SM_TRACE(1);
                     if (i == p.window) {
                         // start-up window: the TMA unit works on all of its outstanding copies at once, so the first
@@ -452,7 +441,7 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         // ===== publisher: releases the partial of every contributor segment that is not the CTA's last one while
         //       the stream runs on (a segment that reaches the tile's last step makes this CTA the reducer: no release) =====
         while (walk.next(tile, s0, s1, final_seg)) {
-            if (final_seg || s1 == S || SM_DBG(p, 4)) continue;
+            if (final_seg || s1 == S) continue;
             asm volatile("bar.sync 2, 160;" ::: "memory");   // the 4 output warps have stored the partial
             if (lane == 0) sm_contribute(counters, tile);
         }
@@ -479,7 +468,6 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
         const uint32_t xsum0 = (uint32_t)(NB * G::kBlk * 1024 + (blk * 8 + m_first) * 4);
         const ACT* const xrow0 = x + (size_t)m_first * (size_t)p.K + cc * 8;
         const size_t row_step = (size_t)kMStep * (size_t)p.K;
-        if (SM_DBG(p, 2)) return;
         // Rows past M are zero in every slot, for ever: written once, here (ordered before the consumers' reads by the
         // first xfull arrive of this thread).
         for (uint32_t o = (uint32_t)(32 * xw + lane) * 16u; o < (uint32_t)p.XR * p.x_slot_bytes; o += 32u * kSmXWarps * 16u)
@@ -573,7 +561,6 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
 #pragma unroll
     for (int sl = 0; sl < 2; ++sl) { rows[sl][0] = (2 * rg + sl) * 16 + sm_row_of<BITS>(gid); rows[sl][1] = rows[sl][0] + 8; }
 
-    const bool do_compute = !SM_DBG(p, 1), do_x = !SM_DBG(p, 2), do_epi = !SM_DBG(p, 4), do_wait = !SM_DBG(p, 8);
     // Absolute shared-memory addresses of this thread's words in slot 0 (rows + 8 / + 16 keep the swizzle phase, so
     // every other address of a stage is one of these plus an immediate).  Made opaque so that they live in registers:
     // ptxas otherwise rematerialises the lane / warp arithmetic inside the stage loop.
@@ -624,152 +611,150 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
     if (tid == 0) SM_TRACE(5);
     while (walk.next(tile, s0, s1, final_seg)) {
         for (int step = s0; step < s1; ++step) {
-            if (do_wait) sm_bar_wait(full_bar(wslot), wph);
+            sm_bar_wait(full_bar(wslot), wph);
 #ifdef QUANTA_SMALL_TRACE
             if (tid == 0 && tr_unit == 0) SM_TRACE(27);
 #endif
-            if (do_x) sm_bar_wait(xfull_bar(xs_cur), xph);
+            sm_bar_wait(xfull_bar(xs_cur), xph);
 #ifdef QUANTA_SMALL_TRACE
             if (tid == 0 && tr_unit == 0) SM_TRACE(28);
 #endif
 
-            if (do_compute) {
-                const uint32_t st_off = (uint32_t)wslot * G::kStageBytes, x_off = (uint32_t)xs_cur * x_slot_bytes;
-                // scales / zero-points of the warp's blocks: rows (slab, half), kBpw adjacent blocks each
-                // (M <= 8: both blocks in one 8-byte read up front; M > 8: per block, late — registers)
-                constexpr bool kParamsUpFront = NB == 1;
-                float sc[2][2][G::kBpw], zc[2][2][G::kBpw];
+            const uint32_t st_off = (uint32_t)wslot * G::kStageBytes, x_off = (uint32_t)xs_cur * x_slot_bytes;
+            // scales / zero-points of the warp's blocks: rows (slab, half), kBpw adjacent blocks each
+            // (M <= 8: both blocks in one 8-byte read up front; M > 8: per block, late — registers)
+            constexpr bool kParamsUpFront = NB == 1;
+            float sc[2][2][G::kBpw], zc[2][2][G::kBpw];
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl)
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    if (!kParamsUpFront) break;
+                    const uint32_t sa = s_base + st_off + (uint32_t)(sl * 16 + h * 8) * kRowPitch;
+                    if (G::kBpw == 2) {
+                        const uint2 a = sm_lds64(sa);
+                        sc[sl][h][0] = __uint_as_float(a.x); sc[sl][h][G::kBpw - 1] = __uint_as_float(a.y);
+                        if (!NF4) {
+                            const uint2 z = sm_lds64(sa + G::kParamTile);
+                            zc[sl][h][0] = __uint_as_float(z.x); zc[sl][h][G::kBpw - 1] = __uint_as_float(z.y);
+                        }
+                    } else {
+                        sc[sl][h][0] = sm_lds32(sa);
+                        if (!NF4) zc[sl][h][0] = sm_lds32(sa + G::kParamTile);
+                    }
+                }
+            const float off = BITS == 4 ? T::kOffset : 0.0f;
+#pragma unroll
+            for (int bb = 0; bb < G::kBpw; ++bb) {
+                // ---- every shared-memory read of the block goes out first (ordered asm statements; the
+                //      arithmetic below is free for the compiler to interleave) ----
+                const uint32_t w_cur = w_base[bb] + st_off;
+                uint32_t wraw[2][2][BITS == 4 ? 2 : 4];  // [slab][row half][words]
 #pragma unroll
                 for (int sl = 0; sl < 2; ++sl)
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
-                        if (!kParamsUpFront) break;
-                        const uint32_t sa = s_base + st_off + (uint32_t)(sl * 16 + h * 8) * kRowPitch;
-                        if (G::kBpw == 2) {
-                            const uint2 a = sm_lds64(sa);
-                            sc[sl][h][0] = __uint_as_float(a.x); sc[sl][h][G::kBpw - 1] = __uint_as_float(a.y);
-                            if (!NF4) {
-                                const uint2 z = sm_lds64(sa + G::kParamTile);
-                                zc[sl][h][0] = __uint_as_float(z.x); zc[sl][h][G::kBpw - 1] = __uint_as_float(z.y);
-                            }
+                        const uint32_t wa = w_cur + (uint32_t)(sl * 2048 + h * 1024);
+                        if (BITS == 4) {
+                            const uint2 w = sm_lds64(wa);
+                            wraw[sl][h][0] = w.x; wraw[sl][h][1] = w.y;
                         } else {
-                            sc[sl][h][0] = sm_lds32(sa);
-                            if (!NF4) zc[sl][h][0] = sm_lds32(sa + G::kParamTile);
+                            const uint4 w = sm_lds128(wa);
+                            wraw[sl][h][0] = w.x; wraw[sl][h][1] = w.y; wraw[sl][h][BITS == 4 ? 0 : 2] = w.z; wraw[sl][h][BITS == 4 ? 1 : 3] = w.w;
                         }
                     }
-                const float off = BITS == 4 ? T::kOffset : 0.0f;
+                uint4 xb[NB];                            // the B fragments of two k steps; re-read for k = 2
+                uint2 xs2[NB];
 #pragma unroll
-                for (int bb = 0; bb < G::kBpw; ++bb) {
-                    // ---- every shared-memory read of the block goes out first (ordered asm statements; the
-                    //      arithmetic below is free for the compiler to interleave) ----
-                    const uint32_t w_cur = w_base[bb] + st_off;
-                    uint32_t wraw[2][2][BITS == 4 ? 2 : 4];  // [slab][row half][words]
+                for (int nb = 0; nb < NB; ++nb) {
+                    xb[nb] = sm_lds128(xb_base + x_off + (uint32_t)((nb * G::kBlk + bb) * 1024));
+                    if (!NF4) xs2[nb] = sm_lds64(xs_base0 + x_off + (uint32_t)((nb * G::kBlk + bb) * 32));
+                }
+                // ---- 4 MMAs (K = 16 each) per slab and batch block: k outermost, so that consecutive MMAs
+                //      are independent (2 slabs x NB accumulators) ----
+                float c[2][NB][4];
 #pragma unroll
-                    for (int sl = 0; sl < 2; ++sl)
+                for (int sl = 0; sl < 2; ++sl)
 #pragma unroll
-                        for (int h = 0; h < 2; ++h) {
-                            const uint32_t wa = w_cur + (uint32_t)(sl * 2048 + h * 1024);
-                            if (BITS == 4) {
-                                const uint2 w = sm_lds64(wa);
-                                wraw[sl][h][0] = w.x; wraw[sl][h][1] = w.y;
-                            } else {
-                                const uint4 w = sm_lds128(wa);
-                                wraw[sl][h][0] = w.x; wraw[sl][h][1] = w.y; wraw[sl][h][BITS == 4 ? 0 : 2] = w.z; wraw[sl][h][BITS == 4 ? 1 : 3] = w.w;
-                            }
-                        }
-                    uint4 xb[NB];                            // the B fragments of two k steps; re-read for k = 2
-                    uint2 xs2[NB];
+                    for (int nb = 0; nb < NB; ++nb) { c[sl][nb][0] = c[sl][nb][1] = c[sl][nb][2] = c[sl][nb][3] = 0.0f; }
 #pragma unroll
-                    for (int nb = 0; nb < NB; ++nb) {
-                        xb[nb] = sm_lds128(xb_base + x_off + (uint32_t)((nb * G::kBlk + bb) * 1024));
-                        if (!NF4) xs2[nb] = sm_lds64(xs_base0 + x_off + (uint32_t)((nb * G::kBlk + bb) * 32));
+                for (int k = 0; k < 4; ++k) {
+                    if (k == 2) {
+#pragma unroll
+                        for (int nb = 0; nb < NB; ++nb) xb[nb] = sm_lds128(xb_base + x_off + (uint32_t)((nb * G::kBlk + bb) * 1024 + 512));
                     }
-                    // ---- 4 MMAs (K = 16 each) per slab and batch block: k outermost, so that consecutive MMAs
-                    //      are independent (2 slabs x NB accumulators) ----
-                    float c[2][NB][4];
-#pragma unroll
-                    for (int sl = 0; sl < 2; ++sl)
-#pragma unroll
-                        for (int nb = 0; nb < NB; ++nb) { c[sl][nb][0] = c[sl][nb][1] = c[sl][nb][2] = c[sl][nb][3] = 0.0f; }
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        if (k == 2) {
-#pragma unroll
-                            for (int nb = 0; nb < NB; ++nb) xb[nb] = sm_lds128(xb_base + x_off + (uint32_t)((nb * G::kBlk + bb) * 1024 + 512));
-                        }
-                        uint32_t a[2][4];                    // {row lo, row+8 lo, row hi, row+8 hi}
-#pragma unroll
-                        for (int sl = 0; sl < 2; ++sl) {
-                            if (NF4) {
-                                // word k / 2, bytes 2 (k & 1) and 2 (k & 1) + 1: K-adjacent pairs in natural order
-                                const uint32_t r0 = wraw[sl][0][k >> 1], r1 = wraw[sl][1][k >> 1];
-                                const uint32_t i00 = (k & 1) ? ((r0 >> 9) & 0x7F80u) : ((r0 << 7) & 0x7F80u);
-                                const uint32_t i01 = (k & 1) ? ((r0 >> 17) & 0x7F80u) : ((r0 >> 1) & 0x7F80u);
-                                const uint32_t i10 = (k & 1) ? ((r1 >> 9) & 0x7F80u) : ((r1 << 7) & 0x7F80u);
-                                const uint32_t i11 = (k & 1) ? ((r1 >> 17) & 0x7F80u) : ((r1 >> 1) & 0x7F80u);
-                                a[sl][0] = __float_as_uint(sm_lds32(lut_lane + i00));
-                                a[sl][1] = __float_as_uint(sm_lds32(lut_lane + i10));
-                                a[sl][2] = __float_as_uint(sm_lds32(lut_lane + i01));
-                                a[sl][3] = __float_as_uint(sm_lds32(lut_lane + i11));
-                            } else if (BITS == 4) {
-                                // word k / 2: pairs (n0,n4) (n1,n5) for even k, (n2,n6) (n3,n7) for odd k.  (The shifts stay
-                                // on the ALU pipe: as IMAD.HI they measured 25 % slower, tools/micro/unit_mix.cu.)
-                                const uint32_t w0 = wraw[sl][0][k >> 1] >> (8 * (k & 1)), w1 = wraw[sl][1][k >> 1] >> (8 * (k & 1));
-                                a[sl][0] = sm_and_or(w0, 0x000F000Fu, T::kMagic);
-                                a[sl][1] = sm_and_or(w1, 0x000F000Fu, T::kMagic);
-                                a[sl][2] = sm_and_or(w0 >> 4, 0x000F000Fu, T::kMagic);
-                                a[sl][3] = sm_and_or(w1 >> 4, 0x000F000Fu, T::kMagic);
-                            } else {
-                                uint32_t p0[2], p1[2];
-                                sm_pairs8<ACT>(wraw[sl][0][k], p0); sm_pairs8<ACT>(wraw[sl][1][k], p1);
-                                a[sl][0] = p0[0]; a[sl][1] = p1[0]; a[sl][2] = p0[1]; a[sl][3] = p1[1];
-                            }
-                        }
-#pragma unroll
-                        for (int nb = 0; nb < NB; ++nb) {
-                            const uint4 xv4 = xb[nb];
-                            const uint32_t b0 = (k & 1) ? xv4.z : xv4.x, b1 = (k & 1) ? xv4.w : xv4.y;
-#pragma unroll
-                            for (int sl = 0; sl < 2; ++sl) T::mma(c[sl][nb], a[sl], b0, b1);
-                        }
-                    }
+                    uint32_t a[2][4];                    // {row lo, row+8 lo, row hi, row+8 hi}
 #pragma unroll
                     for (int sl = 0; sl < 2; ++sl) {
-                        if (!kParamsUpFront) {
-#pragma unroll
-                            for (int h = 0; h < 2; ++h) {
-                                const uint32_t sa = s_base + st_off + (uint32_t)(sl * 16 + h * 8) * kRowPitch + (uint32_t)(bb * 4);
-                                sc[sl][h][bb] = sm_lds32(sa);
-                                if (!NF4) zc[sl][h][bb] = sm_lds32(sa + G::kParamTile);
-                            }
-                        }
                         if (NF4) {
-                            // y += abs_max * raw: the table holds the levels themselves, no offset term
-#pragma unroll
-                            for (int nb = 0; nb < NB; ++nb) {
-                                tot[sl][nb][0] = __fmaf_rn(sc[sl][0][bb], c[sl][nb][0], tot[sl][nb][0]);
-                                tot[sl][nb][1] = __fmaf_rn(sc[sl][0][bb], c[sl][nb][1], tot[sl][nb][1]);
-                                tot[sl][nb][2] = __fmaf_rn(sc[sl][1][bb], c[sl][nb][2], tot[sl][nb][2]);
-                                tot[sl][nb][3] = __fmaf_rn(sc[sl][1][bb], c[sl][nb][3], tot[sl][nb][3]);
-                            }
-                            continue;
+                            // word k / 2, bytes 2 (k & 1) and 2 (k & 1) + 1: K-adjacent pairs in natural order
+                            const uint32_t r0 = wraw[sl][0][k >> 1], r1 = wraw[sl][1][k >> 1];
+                            const uint32_t i00 = (k & 1) ? ((r0 >> 9) & 0x7F80u) : ((r0 << 7) & 0x7F80u);
+                            const uint32_t i01 = (k & 1) ? ((r0 >> 17) & 0x7F80u) : ((r0 >> 1) & 0x7F80u);
+                            const uint32_t i10 = (k & 1) ? ((r1 >> 9) & 0x7F80u) : ((r1 << 7) & 0x7F80u);
+                            const uint32_t i11 = (k & 1) ? ((r1 >> 17) & 0x7F80u) : ((r1 >> 1) & 0x7F80u);
+                            a[sl][0] = __float_as_uint(sm_lds32(lut_lane + i00));
+                            a[sl][1] = __float_as_uint(sm_lds32(lut_lane + i10));
+                            a[sl][2] = __float_as_uint(sm_lds32(lut_lane + i01));
+                            a[sl][3] = __float_as_uint(sm_lds32(lut_lane + i11));
+                        } else if (BITS == 4) {
+                            // word k / 2: pairs (n0,n4) (n1,n5) for even k, (n2,n6) (n3,n7) for odd k.  (The shifts stay
+                            // on the ALU pipe: as IMAD.HI they measured 25 % slower, tools/micro/unit_mix.cu.)
+                            const uint32_t w0 = wraw[sl][0][k >> 1] >> (8 * (k & 1)), w1 = wraw[sl][1][k >> 1] >> (8 * (k & 1));
+                            a[sl][0] = sm_and_or(w0, 0x000F000Fu, T::kMagic);
+                            a[sl][1] = sm_and_or(w1, 0x000F000Fu, T::kMagic);
+                            a[sl][2] = sm_and_or(w0 >> 4, 0x000F000Fu, T::kMagic);
+                            a[sl][3] = sm_and_or(w1 >> 4, 0x000F000Fu, T::kMagic);
+                        } else {
+                            uint32_t p0[2], p1[2];
+                            sm_pairs8<ACT>(wraw[sl][0][k], p0); sm_pairs8<ACT>(wraw[sl][1][k], p1);
+                            a[sl][0] = p0[0]; a[sl][1] = p1[0]; a[sl][2] = p0[1]; a[sl][3] = p1[1];
                         }
-                        const float s_0 = sc[sl][0][bb], s_1 = sc[sl][1][bb];
-                        const float z0 = __fmaf_rn(-off, s_0, zc[sl][0][bb]), z1 = __fmaf_rn(-off, s_1, zc[sl][1][bb]);
+                    }
+#pragma unroll
+                    for (int nb = 0; nb < NB; ++nb) {
+                        const uint4 xv4 = xb[nb];
+                        const uint32_t b0 = (k & 1) ? xv4.z : xv4.x, b1 = (k & 1) ? xv4.w : xv4.y;
+#pragma unroll
+                        for (int sl = 0; sl < 2; ++sl) T::mma(c[sl][nb], a[sl], b0, b1);
+                    }
+                }
+#pragma unroll
+                for (int sl = 0; sl < 2; ++sl) {
+                    if (!kParamsUpFront) {
+#pragma unroll
+                        for (int h = 0; h < 2; ++h) {
+                            const uint32_t sa = s_base + st_off + (uint32_t)(sl * 16 + h * 8) * kRowPitch + (uint32_t)(bb * 4);
+                            sc[sl][h][bb] = sm_lds32(sa);
+                            if (!NF4) zc[sl][h][bb] = sm_lds32(sa + G::kParamTile);
+                        }
+                    }
+                    if (NF4) {
+                        // y += abs_max * raw: the table holds the levels themselves, no offset term
 #pragma unroll
                         for (int nb = 0; nb < NB; ++nb) {
-                            const float xs_a = __uint_as_float(xs2[nb].x), xs_b = __uint_as_float(xs2[nb].y);
-                            tot[sl][nb][0] = __fmaf_rn(s_0, c[sl][nb][0], __fmaf_rn(z0, xs_a, tot[sl][nb][0]));
-                            tot[sl][nb][1] = __fmaf_rn(s_0, c[sl][nb][1], __fmaf_rn(z0, xs_b, tot[sl][nb][1]));
-                            tot[sl][nb][2] = __fmaf_rn(s_1, c[sl][nb][2], __fmaf_rn(z1, xs_a, tot[sl][nb][2]));
-                            tot[sl][nb][3] = __fmaf_rn(s_1, c[sl][nb][3], __fmaf_rn(z1, xs_b, tot[sl][nb][3]));
+                            tot[sl][nb][0] = __fmaf_rn(sc[sl][0][bb], c[sl][nb][0], tot[sl][nb][0]);
+                            tot[sl][nb][1] = __fmaf_rn(sc[sl][0][bb], c[sl][nb][1], tot[sl][nb][1]);
+                            tot[sl][nb][2] = __fmaf_rn(sc[sl][1][bb], c[sl][nb][2], tot[sl][nb][2]);
+                            tot[sl][nb][3] = __fmaf_rn(sc[sl][1][bb], c[sl][nb][3], tot[sl][nb][3]);
                         }
+                        continue;
+                    }
+                    const float s_0 = sc[sl][0][bb], s_1 = sc[sl][1][bb];
+                    const float z0 = __fmaf_rn(-off, s_0, zc[sl][0][bb]), z1 = __fmaf_rn(-off, s_1, zc[sl][1][bb]);
+#pragma unroll
+                    for (int nb = 0; nb < NB; ++nb) {
+                        const float xs_a = __uint_as_float(xs2[nb].x), xs_b = __uint_as_float(xs2[nb].y);
+                        tot[sl][nb][0] = __fmaf_rn(s_0, c[sl][nb][0], __fmaf_rn(z0, xs_a, tot[sl][nb][0]));
+                        tot[sl][nb][1] = __fmaf_rn(s_0, c[sl][nb][1], __fmaf_rn(z0, xs_b, tot[sl][nb][1]));
+                        tot[sl][nb][2] = __fmaf_rn(s_1, c[sl][nb][2], __fmaf_rn(z1, xs_a, tot[sl][nb][2]));
+                        tot[sl][nb][3] = __fmaf_rn(s_1, c[sl][nb][3], __fmaf_rn(z1, xs_b, tot[sl][nb][3]));
                     }
                 }
             }
             // every lane's reads of the stage have been issued (and, in program order, consumed) above
             __syncwarp();
-            if (lane == 0) { sm_bar_arrive(empty_bar(wslot)); if (do_x) sm_bar_arrive(xempty_bar(xs_cur)); }
+            if (lane == 0) { sm_bar_arrive(empty_bar(wslot)); sm_bar_arrive(xempty_bar(xs_cur)); }
             if (++wslot == ring) { wslot = 0; wph ^= 1u; }
             if (++xs_cur == xring) { xs_cur = 0; xph ^= 1u; }
 #ifdef QUANTA_SMALL_TRACE
@@ -777,87 +762,85 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
 #endif
         }
         if (tid == 0) SM_TRACE(6);
-        if (do_epi) {
-            asm volatile("griddepcontrol.wait;" ::: "memory");   // the first global accesses of the consumers follow
-            // ===== end of this CTA's segment [s0, s1) of `tile`: the 4 K quarters meet in shared memory =====
-            const bool whole = s0 == 0 && s1 == S;
-            const uint32_t red = smem + p.red_off + (uint32_t)(rg * (2 * NB * 4) * 128 + lane * 4);
-            const uint32_t red_group = (uint32_t)(4 * 2 * NB * 4 * 128);
-            if (kq > 0) {
+        asm volatile("griddepcontrol.wait;" ::: "memory");   // the first global accesses of the consumers follow
+        // ===== end of this CTA's segment [s0, s1) of `tile`: the 4 K quarters meet in shared memory =====
+        const bool whole = s0 == 0 && s1 == S;
+        const uint32_t red = smem + p.red_off + (uint32_t)(rg * (2 * NB * 4) * 128 + lane * 4);
+        const uint32_t red_group = (uint32_t)(4 * 2 * NB * 4 * 128);
+        if (kq > 0) {
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl)
+#pragma unroll
+                for (int nb = 0; nb < NB; ++nb)
+#pragma unroll
+                    for (int q = 0; q < 4; ++q)
+                        sm_sts32(red + (uint32_t)(kq - 1) * red_group + (uint32_t)(((sl * NB + nb) * 4 + q) * 128), tot[sl][nb][q]);
+        }
+        sm_cons_sync();
+        if (tid == 0) SM_TRACE(29);
+        const int n0 = tile * kSmRows;
+        if (kq == 0) {
+            // tot[sl][nb][q]: feature n0 + rows[sl][q >> 1], batch row 8 nb + 2 tig + (q & 1)
+#pragma unroll
+            for (int sl = 0; sl < 2; ++sl)
+#pragma unroll
+                for (int nb = 0; nb < NB; ++nb)
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) {
+                        const uint32_t ra = red + (uint32_t)(((sl * NB + nb) * 4 + q) * 128);
+                        tot[sl][nb][q] = ((tot[sl][nb][q] + sm_lds32(ra)) + sm_lds32(ra + red_group)) + sm_lds32(ra + 2 * red_group);
+                    }
+            if (whole) {
+#pragma unroll
+                for (int sl = 0; sl < 2; ++sl) {
+#pragma unroll
+                    for (int h = 0; h < 2; ++h) {
+                        const int gn = n0 + rows[sl][h];
+                        const float bv = (bias != nullptr && gn < p.N) ? T::to_float(bias[gn]) : 0.0f;
+#pragma unroll
+                        for (int nb = 0; nb < NB; ++nb)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) {
+                                const int m = 8 * nb + 2 * tig + e;
+                                if (m < p.M && gn < p.N) {
+                                    const ACT v = T::from_float(tot[sl][nb][2 * h + e] + bv);
+                                    for (int o = 0; o < p.n_out; ++o)
+                                        static_cast<ACT*>(p.y[o])[(int64_t)m * p.ldy + p.col0 + gn] = v;
+                                }
+                            }
+                    }
+                }
+            } else {
+                // this CTA's partial slot for the tile: 0 if it is the first tile the CTA touches, else 1;
+                // layout [m][128 features]
+                const int which = (tile == tile0) ? 0 : 1;
+                float* mine = partial + ((size_t)cta * 2 + which) * (size_t)(kSmRows * p.m_pad);
 #pragma unroll
                 for (int sl = 0; sl < 2; ++sl)
 #pragma unroll
                     for (int nb = 0; nb < NB; ++nb)
 #pragma unroll
                         for (int q = 0; q < 4; ++q)
-                            sm_sts32(red + (uint32_t)(kq - 1) * red_group + (uint32_t)(((sl * NB + nb) * 4 + q) * 128), tot[sl][nb][q]);
-            }
-            sm_cons_sync();
-            if (tid == 0) SM_TRACE(29);
-            const int n0 = tile * kSmRows;
-            if (kq == 0) {
-                // tot[sl][nb][q]: feature n0 + rows[sl][q >> 1], batch row 8 nb + 2 tig + (q & 1)
-#pragma unroll
-                for (int sl = 0; sl < 2; ++sl)
-#pragma unroll
-                    for (int nb = 0; nb < NB; ++nb)
-#pragma unroll
-                        for (int q = 0; q < 4; ++q) {
-                            const uint32_t ra = red + (uint32_t)(((sl * NB + nb) * 4 + q) * 128);
-                            tot[sl][nb][q] = ((tot[sl][nb][q] + sm_lds32(ra)) + sm_lds32(ra + red_group)) + sm_lds32(ra + 2 * red_group);
-                        }
-                if (whole) {
-#pragma unroll
-                    for (int sl = 0; sl < 2; ++sl) {
-#pragma unroll
-                        for (int h = 0; h < 2; ++h) {
-                            const int gn = n0 + rows[sl][h];
-                            const float bv = (bias != nullptr && gn < p.N) ? T::to_float(bias[gn]) : 0.0f;
-#pragma unroll
-                            for (int nb = 0; nb < NB; ++nb)
-#pragma unroll
-                                for (int e = 0; e < 2; ++e) {
-                                    const int m = 8 * nb + 2 * tig + e;
-                                    if (m < p.M && gn < p.N) {
-                                        const ACT v = T::from_float(tot[sl][nb][2 * h + e] + bv);
-                                        for (int o = 0; o < p.n_out; ++o)
-                                            static_cast<ACT*>(p.y[o])[(int64_t)m * p.ldy + p.col0 + gn] = v;
-                                    }
-                                }
-                        }
-                    }
-                } else {
-                    // this CTA's partial slot for the tile: 0 if it is the first tile the CTA touches, else 1;
-                    // layout [m][128 features]
-                    const int which = (tile == tile0) ? 0 : 1;
-                    float* mine = partial + ((size_t)cta * 2 + which) * (size_t)(kSmRows * p.m_pad);
-#pragma unroll
-                    for (int sl = 0; sl < 2; ++sl)
-#pragma unroll
-                        for (int nb = 0; nb < NB; ++nb)
-#pragma unroll
-                            for (int q = 0; q < 4; ++q)
-                                __stcg(mine + (8 * nb + 2 * tig + (q & 1)) * kSmRows + rows[sl][q >> 1], tot[sl][nb][q]);
-                    if (!final_seg && s1 != S) {
-                        // a contributor segment with more work behind it: the publisher warp releases it
-                        __syncwarp();
-                        asm volatile("bar.arrive 2, 160;" ::: "memory");
-                    }
+                            __stcg(mine + (8 * nb + 2 * tig + (q & 1)) * kSmRows + rows[sl][q >> 1], tot[sl][nb][q]);
+                if (!final_seg && s1 != S) {
+                    // a contributor segment with more work behind it: the publisher warp releases it
+                    __syncwarp();
+                    asm volatile("bar.arrive 2, 160;" ::: "memory");
                 }
             }
-#pragma unroll
-            for (int sl = 0; sl < 2; ++sl)
-#pragma unroll
-                for (int nb = 0; nb < NB; ++nb) { tot[sl][nb][0] = tot[sl][nb][1] = tot[sl][nb][2] = tot[sl][nb][3] = 0.0f; }
-            if (!whole && s1 == S) red_tile = tile;          // this CTA reduces the tile once its stream has ended
-            if (tid == 0) SM_TRACE(30);
-            sm_cons_sync();
-            if (tid == 0) SM_TRACE(31);                                  // red is reused by the next segment; the partial stores are done
-            if (!whole && final_seg && s1 != S && tid == 0) sm_contribute(counters, tile);
         }
+#pragma unroll
+        for (int sl = 0; sl < 2; ++sl)
+#pragma unroll
+            for (int nb = 0; nb < NB; ++nb) { tot[sl][nb][0] = tot[sl][nb][1] = tot[sl][nb][2] = tot[sl][nb][3] = 0.0f; }
+        if (!whole && s1 == S) red_tile = tile;          // this CTA reduces the tile once its stream has ended
+        if (tid == 0) SM_TRACE(30);
+        sm_cons_sync();
+        if (tid == 0) SM_TRACE(31);                                  // red is reused by the next segment; the partial stores are done
+        if (!whole && final_seg && s1 != S && tid == 0) sm_contribute(counters, tile);
     }
     if (tid == 0) SM_TRACE(7);
-    if (red_tile >= 0 && do_epi) {
+    if (red_tile >= 0) {
         // ===== reducer duty: the other contributors' partials (lower CTA indices) =====
         const unsigned int tu0 = (unsigned int)red_tile * (unsigned int)S;
         const int c_first = sm_cta_of_unit(tu0, p), c_last = (int)cta;
@@ -915,26 +898,9 @@ extern "C" __attribute__((visibility("default"))) int quanta_debug_small_trace(l
 
 // ---- host side --------------------------------------------------------------
 
-struct SmallTuning { int ring; int max_m; int ctas; int dbg; int pdl; int xring; int window; int xw2; };
-static SmallTuning small_tuning() {
-    static const SmallTuning t = []() {
-        SmallTuning v{0, 16, 0, 0, 1, 0, kSmStartWindow, 1};
-        if (const char* e = getenv("QUANTA_B200_SMALL_RING")) { int s = atoi(e); if (s >= 2 && s <= kSmMaxRing) v.ring = s; }
-        if (const char* e = getenv("QUANTA_B200_SMALL_MAX_M")) { int m = atoi(e); if (m >= 0 && m <= 16) v.max_m = m; }
-        if (const char* e = getenv("QUANTA_B200_SMALL_CTAS")) { int c = atoi(e); if (c >= 1 && c <= kNumSMs) v.ctas = c; }
-        if (const char* e = getenv("QUANTA_B200_SMALL_DBG")) v.dbg = atoi(e);
-        if (const char* e = getenv("QUANTA_B200_SMALL_PDL")) v.pdl = atoi(e) != 0;
-        if (const char* e = getenv("QUANTA_B200_SMALL_XRING")) { int s = atoi(e); if (s >= 2 && s <= kSmMaxXRing) v.xring = s; }
-        if (const char* e = getenv("QUANTA_B200_SMALL_XW2")) v.xw2 = atoi(e) != 0;
-        if (const char* e = getenv("QUANTA_B200_SMALL_WINDOW")) { int s = atoi(e); if (s >= 1 && s <= kSmMaxRing) v.window = s; }
-        return v;
-    }();
-    return t;
-}
-
 // The small-batch kernel serves M <= 16 with blockwise-64 parameters on K % 256 == 0.
 bool gemm_small_eligible(int64_t M, int64_t N, int64_t K, int64_t block, const void* scale, const void* zp) {
-    if (M > small_tuning().max_m || block != 64 || (K % kSmKGran) != 0) return false;
+    if (M > kSmMaxM || block != 64 || (K % kSmKGran) != 0) return false;
     if ((reinterpret_cast<uintptr_t>(scale) | reinterpret_cast<uintptr_t>(zp)) & 15) return false;
     const int64_t n_tiles = (N + kSmRows - 1) / kSmRows;
     if (n_tiles > kSmCounterBytes / 4) return false;
@@ -968,29 +934,14 @@ static int gemm_small_launch_nb(const ACT* x, const uint8_t* wq, const float* sc
     if (reinterpret_cast<uintptr_t>(x) & 15) return QUANTA_EINVAL;          // 16-byte activation loads
     p.S = (int)((K + G::kStepK - 1) / G::kStepK);
     p.U = (unsigned int)p.n_tiles * (unsigned int)p.S;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    int sms = kNumSMs;
-    {
-        static int cached[64] = {0};
-        if (dev >= 0 && dev < 64) {
-            if (cached[dev] == 0) {
-                int n = 0;
-                if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = kNumSMs;
-                cached[dev] = n < kNumSMs ? n : kNumSMs;     // partial slots are sized for kNumSMs
-            }
-            sms = cached[dev];
-        }
-    }
+    const int sms = device_sm_count();
     // How many CTAs.  An even cut of the unit range over all SMs streams for the shortest time but ends on the
     // stream-K hand-over (partial stores, release, acquire, fix-up: ~2.5 stage times at M <= 8, more for wider partials)
     // and gives most CTAs two segments; k CTAs per row tile (k = 1: whole tiles, no hand-over at all) stream longer and
     // finish sooner when the tile count is close to a divisor of the SM count.  Costs in stage times, fitted to
     // 4096 x 14336 (32 tiles) and 14336 x 4096 (112 tiles: 11.3 us with one CTA per tile, 12.3 us with 148 ranges).
     int n_cta = (int)(p.U < (unsigned int)sms ? p.U : (unsigned int)sms);
-    if (small_tuning().ctas) {
-        n_cta = small_tuning().ctas < n_cta ? small_tuning().ctas : n_cta;
-    } else if (p.n_tiles <= sms) {
+    if (p.n_tiles <= sms) {
         // Costs of the two endings in stage times, fitted to measurements (W4, stage = 0.9 us at M <= 8, 1.3 us above):
         // an even cut ends on the hand-over AND gives most CTAs two segments; k CTAs per tile end on the hand-over only
         // (k > 1) or on nothing (k = 1).  They are fixed times, so they shrink in stage units as the stage grows (8-bit).
@@ -1015,15 +966,14 @@ static int gemm_small_launch_nb(const ACT* x, const uint8_t* wq, const float* sc
     // The activation ring is sized first — 4 slots for M <= 8, 3 for M > 8 (measured at 4096 x 14336, M = 16: 3 slots +
     // 3 stages 17.0 us, 2 + 4: 19.3, 4 + 3: 18.4; its staging warps prefetch only one unit in registers there) — and
     // the weight ring gets what is left.
-    const int xring = small_tuning().xring ? small_tuning().xring : (NB == 1 ? kSmMaxXRing : 3);
+    const int xring = NB == 1 ? kSmMaxXRing : 3;
     const uint32_t lut_bytes = NF4 ? kSmLutBytes : 0u;
     int ring = (int)((budget - (uint32_t)xring * p.x_slot_bytes - red_bytes - bar_bytes - lut_bytes) / G::kStageBytes);
     if (ring > kSmMaxRing) ring = kSmMaxRing;
-    if (small_tuning().ring && small_tuning().ring < ring) ring = small_tuning().ring;
-    if (ring < 2 || xring < 2) return QUANTA_EUNSUPPORTED;
+    if (ring < 2) return QUANTA_EUNSUPPORTED;
     p.R = ring;
     p.XR = xring;
-    p.window = small_tuning().window < ring ? small_tuning().window : ring;
+    p.window = kSmStartWindow < ring ? kSmStartWindow : ring;
     const uint32_t x_bytes = (uint32_t)xring * p.x_slot_bytes;
     p.x_off = (uint32_t)ring * G::kStageBytes;
     p.lut_off = p.x_off + x_bytes;
@@ -1031,7 +981,6 @@ static int gemm_small_launch_nb(const ACT* x, const uint8_t* wq, const float* sc
     p.bar_off = p.red_off + red_bytes;
     const int smem = (int)(p.bar_off + bar_bytes);
     p.ldy = (int)ldy; p.col0 = (int)col0; p.n_out = n_out;
-    p.dbg = small_tuning().dbg;
     bool aligned8 = true;
     for (int o = 0; o < kSmMaxOut; ++o) {
         p.y[o] = o < n_out ? ys[o] : nullptr;
@@ -1069,7 +1018,7 @@ static int gemm_small_launch_nb(const ACT* x, const uint8_t* wq, const float* sc
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = small_tuning().pdl ? 1 : 0;
+    cfg.numAttrs = 1;
     cudaError_t e = cudaLaunchKernelEx(&cfg, kern, tmap_w, tmap_s, tmap_z, x, bias, counters, partial, p);
     return cuda_status(e != cudaSuccess ? e : cudaGetLastError());
 }
@@ -1078,7 +1027,7 @@ template <typename ACT, int BITS>
 int gemm_small_launch(const ACT* x, const uint8_t* wq, const float* scale, const float* zp, const ACT* bias, void* const* ys,
                       int n_out, int64_t ldy, int64_t col0, int64_t M, int64_t N, int64_t K, void* workspace, size_t ws_bytes,
                       cudaStream_t st, int nf4, const PeerSync* sync) {
-    const bool one = M == 1 && small_tuning().xw2;           // a single batch row: two staging warps (see sm_threads)
+    const bool one = M == 1;                                 // a single batch row: two staging warps (see sm_threads)
     if (nf4) {
         // 4-bit codes index the NF4 table, `scale` holds abs_max per block, `zp` is not read
         if (BITS != 4) return QUANTA_EINVAL;

@@ -1,11 +1,9 @@
 // Host-side helpers shared by every launcher: the tensor-map encoder (with a cache), the per-device
-// dynamic-shared-memory attribute, environment switches read once.
+// dynamic-shared-memory attribute, the SM count.
 #include "common.cuh"
 
-#include <cstdlib>
 #include <cstring>
 #include <mutex>
-#include <string>
 #include <unordered_map>
 
 namespace quanta {
@@ -92,16 +90,16 @@ int ensure_dynamic_smem(const void* func, int bytes) {
     return 0;
 }
 
-int env_int(const char* name, int fallback) {
-    static std::mutex mu;
-    static std::unordered_map<std::string, int> cache;
-    std::lock_guard<std::mutex> lock(mu);
-    auto it = cache.find(name);
-    if (it != cache.end()) return it->second;
-    const char* e = getenv(name);
-    const int v = (e && *e) ? atoi(e) : fallback;
-    cache.emplace(name, v);
-    return v;
+int device_sm_count() {
+    static int cached[64] = {0};
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return kNumSMs;
+    if (cached[dev] == 0) {
+        int n = 0;
+        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = kNumSMs;
+        cached[dev] = n < kNumSMs ? n : kNumSMs;
+    }
+    return cached[dev];
 }
 
 }  // namespace quanta

@@ -17,7 +17,6 @@
 //                               outlier columns on the CUDA cores and stores y
 #include "common.cuh"
 
-#include <cstdlib>
 #include <type_traits>
 
 namespace quanta {
@@ -459,7 +458,6 @@ static int outlier_launch(const ACT* x, const int8_t* qw, const float* cw, float
     if (nk_all >= 64 && (size_t)M * (size_t)N * 4 <= kOAccBytes && tiles * 4 <= (int64_t)kOCounterBytes) {
         while (splits < 16 && tiles * (splits * 2) <= kNumSMs && nk_all / (splits * 2) >= 4) splits *= 2;
     }
-    if (env_int("QUANTA_B200_OUTLIER_SPLITS", 0) == 1) splits = 1;
     p.splits = splits;
     if (splits > 1 || M > 64) {
         size_t clear = (size_t)K * 4;

@@ -12,7 +12,6 @@
 #include "common.cuh"
 
 #include <cstdio>
-#include <cstdlib>
 
 namespace quanta {
 
@@ -304,7 +303,7 @@ __global__ void dim0_earlyout_params_kernel(int64_t cols, float* scale_out, floa
 }
 
 // --------------------------------------------------------------------------
-// 2. the streaming TMA kernel (BLOCK and TENSOR modes)
+// 2. the streaming TMA kernel (BLOCK mode)
 // --------------------------------------------------------------------------
 constexpr int kRowElems = 32;          // elements owned by one consumer thread
 constexpr int kTileRows = 256;         // rows (= consumer threads) per TMA tile
@@ -383,21 +382,70 @@ __device__ __noinline__ float slow_row_codes(const float* v, float mn, float mx,
     return p.scale;
 }
 
-template <typename T, int BITS, bool PACK, int CONV, bool BLOCKWISE, bool DYN>
-__global__ void __launch_bounds__(kTmaThreads, 2)
-quantize_rows_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t n_rows, int log2_lanes_per_block,
-                         uint8_t* __restrict__ q_out, float* __restrict__ scale_out, float* __restrict__ zp_out,
-                         const float* ws, int nparts) {
+// The tensors of one launch: a single tensor (quantize_rows_tma_kernel) or up to kMultiMax of them
+// (quantize_rows_tma_multi_kernel).  Quantizing a model is hundreds of independent matrices; one launch
+// per matrix pays a prologue (barrier setup, tensor-map fetch, first-tile latency) and a tail each
+// time.  The multi-tensor launch lets them share one grid: the tile index space is the concatenation
+// of the tensors' tiles, the descriptors ride in the kernel parameters (tensor maps included), and
+// cluster launch control balances the lot.
+constexpr int kMultiMax = 16;
+struct MultiArgs {
+    CUtensorMap maps[kMultiMax];
+    int64_t n_rows[kMultiMax];
+    uint8_t* q[kMultiMax];
+    float* scale[kMultiMax];
+    float* zp[kMultiMax];
+    int tile_base[kMultiMax + 1];     // first global tile of tensor i; [count] = total
+    int count;
+};
+
+// Both describe their tensors to quantize_rows_stream the same way: locate() maps a tile of the
+// launch to (tensor ti, tile within it).
+struct RowsOne {
+    static constexpr bool kMulti = false;
+    const CUtensorMap* tmap;
+    int64_t n_rows;
+    uint8_t* q_out;
+    float* scale_out;
+    float* zp_out;
+    __device__ __forceinline__ int n_tiles() const { return (int)((n_rows + kTileRows - 1) / kTileRows); }
+    __device__ __forceinline__ int locate(int g, int& ti) const { ti = 0; return g; }
+    __device__ __forceinline__ const CUtensorMap* map(int) const { return tmap; }
+    __device__ __forceinline__ int64_t rows(int) const { return n_rows; }
+    __device__ __forceinline__ uint8_t* q(int) const { return q_out; }
+    __device__ __forceinline__ float* scale(int) const { return scale_out; }
+    __device__ __forceinline__ float* zp(int) const { return zp_out; }
+};
+struct RowsMulti {
+    static constexpr bool kMulti = true;
+    const MultiArgs& a;
+    __device__ __forceinline__ int n_tiles() const { return a.tile_base[a.count]; }
+    __device__ __forceinline__ int locate(int g, int& ti) const {
+        ti = 0;
+        while (ti + 1 < a.count && g >= a.tile_base[ti + 1]) ++ti;
+        return g - a.tile_base[ti];
+    }
+    __device__ __forceinline__ const CUtensorMap* map(int ti) const { return &a.maps[ti]; }
+    __device__ __forceinline__ int64_t rows(int ti) const { return a.n_rows[ti]; }
+    __device__ __forceinline__ uint8_t* q(int ti) const { return a.q[ti]; }
+    __device__ __forceinline__ float* scale(int ti) const { return a.scale[ti]; }
+    __device__ __forceinline__ float* zp(int ti) const { return a.zp[ti]; }
+};
+
+// Blockwise (convention A) row stream, one CTA per tile of the launch: resident CTAs steal the
+// not-yet-launched ones (cluster launch control).
+template <typename T, int BITS, bool PACK, typename Src>
+__device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_lanes_per_block) {
     using RL = RowLayout<T>;
     extern __shared__ uint8_t smem_raw[];
     __shared__ uint64_t full_bar[kStages], empty_bar[kStages], clc_bar;
     __shared__ uint32_t dep_scratch[kTmaThreads / 32];           // see mbar_arrive_after_loads
     __shared__ __align__(16) uint4 clc_resp;
-    __shared__ int tile_of_stage[kStages];
+    __shared__ int tile_of_stage[kStages], tens_of_stage[kStages];
 
     const uint32_t smem = (smem_u32(smem_raw) + 1023u) & ~1023u;       // SWIZZLE_128B atoms are 1 KB
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int n_tiles = (int)((n_rows + kTileRows - 1) / kTileRows);
+    const int n_tiles = src.n_tiles();
 
     if (tid == 0) {
 #pragma unroll
@@ -411,76 +459,42 @@ quantize_rows_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t n_row
     if (warp == kConsumerWarps) {
         // ===== producer warp: one lane streams tiles into the ring =====
         if (lane == 0) {
-            prefetch_tensormap(&tmap);
+            if (!Src::kMulti) prefetch_tensormap(src.map(0));
             const uint64_t policy = policy_evict_first();
-            int cta = blockIdx.x;          // DYN: this CTA's own tile first, then stolen ones
+            int cta = blockIdx.x;          // this CTA's own tile first, then stolen ones
             uint32_t clc_phase = 0;
             for (int i = 0;; ++i) {
                 const int s = i % kStages;
                 const uint32_t ph = (i / kStages) & 1;
                 mbar_wait(&empty_bar[s], ph ^ 1);
                 const bool live = cta >= 0 && cta < n_tiles;
-                const int t = !live ? -1 : (BLOCKWISE ? cta : n_tiles - 1 - cta);   // TENSOR pass 2: newest-in-L2 first
+                if (!live) { tile_of_stage[s] = -1; mbar_arrive(&full_bar[s]); break; }
+                int ti;
+                const int t = src.locate(cta, ti);
                 tile_of_stage[s] = t;
-                if (!live) { mbar_arrive(&full_bar[s]); break; }
+                if (Src::kMulti) tens_of_stage[s] = ti;
                 mbar_arrive_expect_tx(&full_bar[s], RL::kTileBytes);
-                tma_load_2d_addr(smem + s * RL::kTileBytes, &tmap, smem_u32(&full_bar[s]), 0, t * kTileRows, policy);
-                if (DYN) {
-                    mbar_arrive_expect_tx(&clc_bar, 16);
-                    clc_try_cancel(smem_u32(&clc_resp), smem_u32(&clc_bar));
-                    mbar_wait(&clc_bar, clc_phase);
-                    clc_phase ^= 1;
-                    cta = clc_read(smem_u32(&clc_resp));
-                } else {
-                    cta += gridDim.x;
-                }
+                tma_load_2d_addr(smem + s * RL::kTileBytes, src.map(ti), smem_u32(&full_bar[s]), 0, t * kTileRows, policy);
+                mbar_arrive_expect_tx(&clc_bar, 16);
+                clc_try_cancel(smem_u32(&clc_resp), smem_u32(&clc_bar));
+                mbar_wait(&clc_bar, clc_phase);
+                clc_phase ^= 1;
+                cta = clc_read(smem_u32(&clc_resp));
             }
         }
         return;
     }
 
     // ===== consumers: thread `tid` owns row `tid` of every tile =====
-    constexpr float L = BITS == 8 ? 255.0f : 15.0f;
-    constexpr float Q = BITS == 8 ? 127.0f : 7.0f;
-    ElemParams gp{0.f, 1.f, 0.f};
-    bool early = false;
-    if (!BLOCKWISE) {
-        // TENSOR mode: every CTA reduces the per-CTA partial min/max of pass 1 itself
-        // (a few KB from L2) instead of waiting for a separate single-CTA finalize launch.
-        __shared__ float red_mn[kConsumerWarps], red_mx[kConsumerWarps];
-        const float* pmin = ws + kWsHeaderFloats + 64;
-        const float* pmax = pmin + kMaxPartialCtas;
-        float mn = pmin[0], mx = pmax[0];
-        for (int k = tid; k < nparts; k += kTileRows) { mn = min_nan(mn, pmin[k]); mx = max_nan(mx, pmax[k]); }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            mn = min_nan(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-            mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        }
-        if (lane == 0) { red_mn[warp] = mn; red_mx[warp] = mx; }
-        asm volatile("bar.sync 1, %0;" ::"n"(kTileRows) : "memory");      // consumers only
-#pragma unroll
-        for (int w = 0; w < kConsumerWarps; ++w) { mn = min_nan(mn, red_mn[w]); mx = max_nan(mx, red_mx[w]); }
-        float sc, z, r; bool close;
-        group_params<CONV>(mn, mx, BITS, &sc, &z, &r, &close);
-        early = (CONV != kConvA) && close;
-        if (early) { sc = 1.0f; z = mn; }                 // cpu/quantization.py:38-39
-        gp.s = sc; gp.a = z; gp.r = r;
-        if (blockIdx.x == 0 && tid == 0) {                // publish for the caller and the tail kernel
-            scale_out[0] = sc; zp_out[0] = z;
-            const_cast<float*>(ws)[kWsHeaderFloats] = r;
-            reinterpret_cast<int*>(const_cast<float*>(ws))[0] = early ? 1 : 0;
-        }
-    }
     const int lpb_mask = (1 << log2_lanes_per_block) - 1;
     const uint32_t row_off = tid * RL::kRowBytes;
-
     for (int i = 0;; ++i) {
         const int s = i % kStages;
         const uint32_t ph = (i / kStages) & 1;
         mbar_wait(&full_bar[s], ph);
         const int t = *reinterpret_cast<volatile int*>(&tile_of_stage[s]);
         if (t < 0) break;
+        const int ti = Src::kMulti ? *reinterpret_cast<volatile int*>(&tens_of_stage[s]) : 0;
 
         float v[kRowElems];
         const uint32_t row = smem + s * RL::kTileBytes + row_off;
@@ -499,87 +513,82 @@ quantize_rows_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t n_row
         __syncwarp();
         if (lane == 0) mbar_arrive_after_loads(&empty_bar[s], row_dep<T>(v), &dep_scratch[warp]);     // stage can be refilled while we compute
 
-        const int64_t grow = (int64_t)t * kTileRows + tid;      // global row
-        const bool row_ok = grow < n_rows;
+        const int64_t grow = (int64_t)t * kTileRows + tid;      // row within the tensor
+        const bool row_ok = grow < src.rows(ti);
         uint32_t u[kRowElems];
-
-        if (BLOCKWISE) {
-            float m0[4], m1[4];
+        float m0[4], m1[4];
 #pragma unroll
-            for (int k = 0; k < 4; ++k) { m0[k] = v[k]; m1[k] = v[k]; }
+        for (int k = 0; k < 4; ++k) { m0[k] = v[k]; m1[k] = v[k]; }
 #pragma unroll
-            for (int k = 4; k < kRowElems; ++k) { m0[k & 3] = min_nan(m0[k & 3], v[k]); m1[k & 3] = max_nan(m1[k & 3], v[k]); }
-            float mn = min_nan(min_nan(m0[0], m0[1]), min_nan(m0[2], m0[3]));
-            float mx = max_nan(max_nan(m1[0], m1[1]), max_nan(m1[2], m1[3]));
-            for (int o = 1; o <= lpb_mask; o <<= 1) {
-                mn = min_nan(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-                mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-            }
-            // quantization.py:195-196 / :205: degenerate range rule, scale = range / L
-            const float mx2 = (mx == mn) ? __fadd_rn(mn, 1e-6f) : mx;
-            const float range = __fsub_rn(mx2, mn);
-            // range in [2^-50, 2^50] (false for NaN/inf): constant-reciprocal divide and
-            // hoisted-reciprocal quotients are exact, and x in [mn, mx] makes the clamp a no-op
-            const bool fast = range >= 8.881784197001252e-16f && range <= 1125899906842624.0f;
-            float scale;
-            if (__all_sync(0xffffffffu, fast)) {
-                scale = div_by_levels<BITS>(range);
-                const float rcp = __frcp_rn(scale);
-                const float nscale = -scale;
-#pragma unroll
-                for (int k = 0; k < kRowElems; ++k) {
-                    const float a = __fsub_rn(v[k], mn);
-                    const float q0 = __fmul_rn(a, rcp);
-                    const float r = __fmaf_rn(nscale, q0, a);
-                    u[k] = __float_as_uint(__fadd_rn(__fmaf_rn(rcp, r, q0), kMagic));
-                }
-            } else {
-                // copies keep v[] / u[] in registers on the hot path (only these temporaries live on the stack)
-                float vs[kRowElems];
-                uint32_t us[kRowElems];
-#pragma unroll
-                for (int k = 0; k < kRowElems; ++k) vs[k] = v[k];
-                scale = slow_row_codes<BITS>(vs, mn, mx, us);
-#pragma unroll
-                for (int k = 0; k < kRowElems; ++k) u[k] = us[k];
-            }
-            if (row_ok && (lane & lpb_mask) == 0) {
-                const int64_t b = grow >> log2_lanes_per_block;
-                scale_out[b] = scale;
-                zp_out[b] = mn;
-            }
-        } else if (CONV == kConvA && gp.r != 0.0f) {
-            const float nscale = -gp.s;
+        for (int k = 4; k < kRowElems; ++k) { m0[k & 3] = min_nan(m0[k & 3], v[k]); m1[k & 3] = max_nan(m1[k & 3], v[k]); }
+        float mn = min_nan(min_nan(m0[0], m0[1]), min_nan(m0[2], m0[3]));
+        float mx = max_nan(max_nan(m1[0], m1[1]), max_nan(m1[2], m1[3]));
+        for (int o = 1; o <= lpb_mask; o <<= 1) {
+            mn = min_nan(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+            mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+        }
+        // quantization.py:195-196 / :205: degenerate range rule, scale = range / L
+        const float mx2 = (mx == mn) ? __fadd_rn(mn, 1e-6f) : mx;
+        const float range = __fsub_rn(mx2, mn);
+        // range in [2^-50, 2^50] (false for NaN/inf): constant-reciprocal divide and
+        // hoisted-reciprocal quotients are exact, and x in [mn, mx] makes the clamp a no-op
+        const bool fast = range >= 8.881784197001252e-16f && range <= 1125899906842624.0f;
+        float scale;
+        if (__all_sync(0xffffffffu, fast)) {
+            scale = div_by_levels<BITS>(range);
+            const float rcp = __frcp_rn(scale);
+            const float nscale = -scale;
 #pragma unroll
             for (int k = 0; k < kRowElems; ++k) {
-                const float a = __fsub_rn(v[k], gp.a);
-                const float q0 = __fmul_rn(a, gp.r);
-                const float r = __fmaf_rn(nscale, q0, a);
-                // rows past the end of the tensor are zero-filled by TMA: clamp keeps them harmless
-                u[k] = code_bits(__fmaf_rn(gp.r, r, q0), L);
+                const float d = __fsub_rn(v[k], mn);
+                const float q0 = __fmul_rn(d, rcp);
+                const float r = __fmaf_rn(nscale, q0, d);
+                u[k] = __float_as_uint(__fadd_rn(__fmaf_rn(rcp, r, q0), kMagic));
             }
         } else {
+            // copies keep v[] / u[] in registers on the hot path (only these temporaries live on the stack)
+            float vs[kRowElems];
+            uint32_t us[kRowElems];
 #pragma unroll
-            for (int k = 0; k < kRowElems; ++k) u[k] = elem_code_bits<CONV, false>(v[k], gp, L, Q);
+            for (int k = 0; k < kRowElems; ++k) vs[k] = v[k];
+            scale = slow_row_codes<BITS>(vs, mn, mx, us);
+#pragma unroll
+            for (int k = 0; k < kRowElems; ++k) u[k] = us[k];
         }
-
+        if (row_ok && (lane & lpb_mask) == 0) {
+            const int64_t b = grow >> log2_lanes_per_block;
+            src.scale(ti)[b] = scale;
+            src.zp(ti)[b] = mn;
+        }
         if (row_ok) {
             if (BITS == 4 && PACK) {
                 uint4 o;
-                o.x = pack_nibbles8<CONV>(u + 0);  o.y = pack_nibbles8<CONV>(u + 8);
-                o.z = pack_nibbles8<CONV>(u + 16); o.w = pack_nibbles8<CONV>(u + 24);
-                if (early) o = make_uint4(0, 0, 0, 0);
-                __stcs(reinterpret_cast<uint4*>(q_out + grow * 16), o);
+                o.x = pack_nibbles8<kConvA>(u + 0);  o.y = pack_nibbles8<kConvA>(u + 8);
+                o.z = pack_nibbles8<kConvA>(u + 16); o.w = pack_nibbles8<kConvA>(u + 24);
+                __stcs(reinterpret_cast<uint4*>(src.q(ti) + grow * 16), o);
             } else {
                 uint32_t w[8];
 #pragma unroll
-                for (int k = 0; k < 8; ++k) w[k] = early ? 0u : pack_bytes4<CONV, BITS>(u[4 * k], u[4 * k + 1], u[4 * k + 2], u[4 * k + 3]);
-                uint4* dst = reinterpret_cast<uint4*>(q_out + grow * 32);
+                for (int k = 0; k < 8; ++k) w[k] = pack_bytes4<kConvA, BITS>(u[4 * k], u[4 * k + 1], u[4 * k + 2], u[4 * k + 3]);
+                uint4* dst = reinterpret_cast<uint4*>(src.q(ti) + grow * 32);
                 __stcs(dst, make_uint4(w[0], w[1], w[2], w[3]));
                 __stcs(dst + 1, make_uint4(w[4], w[5], w[6], w[7]));
             }
         }
     }
+}
+
+template <typename T, int BITS, bool PACK>
+__global__ void __launch_bounds__(kTmaThreads, 2)
+quantize_rows_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t n_rows, int log2_lanes_per_block,
+                         uint8_t* __restrict__ q_out, float* __restrict__ scale_out, float* __restrict__ zp_out) {
+    quantize_rows_stream<T, BITS, PACK>(RowsOne{&tmap, n_rows, q_out, scale_out, zp_out}, log2_lanes_per_block);
+}
+
+template <typename T, int BITS, bool PACK>
+__global__ void __launch_bounds__(kTmaThreads, 2)
+quantize_rows_tma_multi_kernel(const __grid_constant__ MultiArgs a, int log2_lanes_per_block) {
+    quantize_rows_stream<T, BITS, PACK>(RowsMulti{a}, log2_lanes_per_block);
 }
 
 // --------------------------------------------------------------------------
@@ -1243,164 +1252,6 @@ quantize_dim0_fused_kernel(const __grid_constant__ CUtensorMap tmap, int64_t row
 }
 
 // --------------------------------------------------------------------------
-// 2b. the same stream over SEVERAL tensors in one launch (blockwise, convention A)
-// --------------------------------------------------------------------------
-// Quantizing a model is hundreds of independent matrices; one launch per matrix pays a
-// prologue (barrier setup, tensor-map fetch, first-tile latency) and a tail each time.  Here up
-// to kMultiMax tensors share one grid: the tile index space is the concatenation of the tensors'
-// tiles, the descriptors ride in the kernel parameters (tensor maps included), and cluster
-// launch control balances the lot.
-constexpr int kMultiMax = 16;
-struct MultiArgs {
-    CUtensorMap maps[kMultiMax];
-    int64_t n_rows[kMultiMax];
-    uint8_t* q[kMultiMax];
-    float* scale[kMultiMax];
-    float* zp[kMultiMax];
-    int tile_base[kMultiMax + 1];     // first global tile of tensor i; [count] = total
-    int count;
-};
-
-template <typename T, int BITS, bool PACK>
-__global__ void __launch_bounds__(kTmaThreads, 2)
-quantize_rows_tma_multi_kernel(const __grid_constant__ MultiArgs a, int log2_lanes_per_block) {
-    using RL = RowLayout<T>;
-    extern __shared__ uint8_t smem_raw[];
-    __shared__ uint64_t full_bar[kStages], empty_bar[kStages], clc_bar;
-    __shared__ uint32_t dep_scratch[kTmaThreads / 32];           // see mbar_arrive_after_loads
-    __shared__ __align__(16) uint4 clc_resp;
-    __shared__ int tile_of_stage[kStages], tens_of_stage[kStages];
-
-    const uint32_t smem = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int n_tiles = a.tile_base[a.count];
-
-    if (tid == 0) {
-#pragma unroll
-        for (int s = 0; s < kStages; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], kConsumerWarps); }
-        mbar_init(&clc_bar, 1);
-        fence_barrier_init();
-    }
-    __syncthreads();
-    pdl_wait();                                            // the set-up above may overlap the previous kernel's tail
-
-    if (warp == kConsumerWarps) {
-        if (lane == 0) {
-            const uint64_t policy = policy_evict_first();
-            int cta = blockIdx.x;
-            uint32_t clc_phase = 0;
-            for (int i = 0;; ++i) {
-                const int s = i % kStages;
-                const uint32_t ph = (i / kStages) & 1;
-                mbar_wait(&empty_bar[s], ph ^ 1);
-                const bool live = cta >= 0 && cta < n_tiles;
-                if (!live) { tile_of_stage[s] = -1; mbar_arrive(&full_bar[s]); break; }
-                int ti = 0;
-                while (ti + 1 < a.count && cta >= a.tile_base[ti + 1]) ++ti;
-                const int t = cta - a.tile_base[ti];
-                tile_of_stage[s] = t;
-                tens_of_stage[s] = ti;
-                mbar_arrive_expect_tx(&full_bar[s], RL::kTileBytes);
-                tma_load_2d_addr(smem + s * RL::kTileBytes, &a.maps[ti], smem_u32(&full_bar[s]), 0, t * kTileRows, policy);
-                mbar_arrive_expect_tx(&clc_bar, 16);
-                clc_try_cancel(smem_u32(&clc_resp), smem_u32(&clc_bar));
-                mbar_wait(&clc_bar, clc_phase);
-                clc_phase ^= 1;
-                cta = clc_read(smem_u32(&clc_resp));
-            }
-        }
-        return;
-    }
-
-    const int lpb_mask = (1 << log2_lanes_per_block) - 1;
-    const uint32_t row_off = tid * RL::kRowBytes;
-    for (int i = 0;; ++i) {
-        const int s = i % kStages;
-        const uint32_t ph = (i / kStages) & 1;
-        mbar_wait(&full_bar[s], ph);
-        const int t = *reinterpret_cast<volatile int*>(&tile_of_stage[s]);
-        if (t < 0) break;
-        const int ti = *reinterpret_cast<volatile int*>(&tens_of_stage[s]);
-
-        float v[kRowElems];
-        const uint32_t row = smem + s * RL::kTileBytes + row_off;
-#pragma unroll
-        for (int j = 0; j < RL::kChunks; ++j) {
-            uint4 c = lds128(row + (RL::swz(tid, j) << 4));
-            if (sizeof(T) == 4) {
-                v[4 * j + 0] = __uint_as_float(c.x); v[4 * j + 1] = __uint_as_float(c.y);
-                v[4 * j + 2] = __uint_as_float(c.z); v[4 * j + 3] = __uint_as_float(c.w);
-            } else {
-                const T* e = reinterpret_cast<const T*>(&c);
-#pragma unroll
-                for (int k = 0; k < 8; ++k) v[8 * j + k] = to_f32(e[k]);
-            }
-        }
-        __syncwarp();
-        if (lane == 0) mbar_arrive_after_loads(&empty_bar[s], row_dep<T>(v), &dep_scratch[warp]);
-
-        const int64_t grow = (int64_t)t * kTileRows + tid;
-        const bool row_ok = grow < a.n_rows[ti];
-        uint32_t u[kRowElems];
-        float m0[4], m1[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) { m0[k] = v[k]; m1[k] = v[k]; }
-#pragma unroll
-        for (int k = 4; k < kRowElems; ++k) { m0[k & 3] = min_nan(m0[k & 3], v[k]); m1[k & 3] = max_nan(m1[k & 3], v[k]); }
-        float mn = min_nan(min_nan(m0[0], m0[1]), min_nan(m0[2], m0[3]));
-        float mx = max_nan(max_nan(m1[0], m1[1]), max_nan(m1[2], m1[3]));
-        for (int o = 1; o <= lpb_mask; o <<= 1) {
-            mn = min_nan(mn, __shfl_xor_sync(0xffffffffu, mn, o));
-            mx = max_nan(mx, __shfl_xor_sync(0xffffffffu, mx, o));
-        }
-        const float mx2 = (mx == mn) ? __fadd_rn(mn, 1e-6f) : mx;
-        const float range = __fsub_rn(mx2, mn);
-        const bool fast = range >= 8.881784197001252e-16f && range <= 1125899906842624.0f;
-        float scale;
-        if (__all_sync(0xffffffffu, fast)) {
-            scale = div_by_levels<BITS>(range);
-            const float rcp = __frcp_rn(scale);
-            const float nscale = -scale;
-#pragma unroll
-            for (int k = 0; k < kRowElems; ++k) {
-                const float d = __fsub_rn(v[k], mn);
-                const float q0 = __fmul_rn(d, rcp);
-                const float r = __fmaf_rn(nscale, q0, d);
-                u[k] = __float_as_uint(__fadd_rn(__fmaf_rn(rcp, r, q0), kMagic));
-            }
-        } else {
-            float vs[kRowElems];
-            uint32_t us[kRowElems];
-#pragma unroll
-            for (int k = 0; k < kRowElems; ++k) vs[k] = v[k];
-            scale = slow_row_codes<BITS>(vs, mn, mx, us);
-#pragma unroll
-            for (int k = 0; k < kRowElems; ++k) u[k] = us[k];
-        }
-        if (row_ok && (lane & lpb_mask) == 0) {
-            const int64_t b = grow >> log2_lanes_per_block;
-            a.scale[ti][b] = scale;
-            a.zp[ti][b] = mn;
-        }
-        if (row_ok) {
-            if (BITS == 4 && PACK) {
-                uint4 o;
-                o.x = pack_nibbles8<kConvA>(u + 0);  o.y = pack_nibbles8<kConvA>(u + 8);
-                o.z = pack_nibbles8<kConvA>(u + 16); o.w = pack_nibbles8<kConvA>(u + 24);
-                __stcs(reinterpret_cast<uint4*>(a.q[ti] + grow * 16), o);
-            } else {
-                uint32_t w[8];
-#pragma unroll
-                for (int k = 0; k < 8; ++k) w[k] = pack_bytes4<kConvA, BITS>(u[4 * k], u[4 * k + 1], u[4 * k + 2], u[4 * k + 3]);
-                uint4* dst = reinterpret_cast<uint4*>(a.q[ti] + grow * 32);
-                __stcs(dst, make_uint4(w[0], w[1], w[2], w[3]));
-                __stcs(dst + 1, make_uint4(w[4], w[5], w[6], w[7]));
-            }
-        }
-    }
-}
-
-// --------------------------------------------------------------------------
 // 3. dim-0 quantize: thread owns 4 columns, walks down the rows
 // --------------------------------------------------------------------------
 template <typename T, int BITS, bool PACK, int CONV>
@@ -1535,74 +1386,28 @@ template <> struct TmaType<float> { static constexpr CUtensorMapDataType v = CU_
 template <> struct TmaType<__half> { static constexpr CUtensorMapDataType v = CU_TENSOR_MAP_DATA_TYPE_FLOAT16; };
 template <> struct TmaType<__nv_bfloat16> { static constexpr CUtensorMapDataType v = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16; };
 
-static int grid_for_tiles(int64_t n_tiles) {
-    int64_t g = (int64_t)kNumSMs * 2;
-    return (int)(n_tiles < g ? n_tiles : g);
-}
-
-static bool use_clc() {
-    static const bool v = []() {
-        const char* e = getenv("QUANTA_B200_STATIC_TILES");      // escape hatch: static round-robin tiles
-        return !(e && e[0] == '1');
-    }();
-    return v;
-}
-
 static int log2_of(int64_t v) {
     int s = 0;
     while ((int64_t(1) << s) < v) ++s;
     return s;
 }
 
-template <typename T, int BITS, bool PACK, int CONV, bool BLOCKWISE, bool DYN>
-static int launch_rows_tma_impl(const CUtensorMap& tmap, int64_t n_rows, int lanes_per_block, uint8_t* q, float* scale,
-                                float* zp, const float* ws, int nparts, cudaStream_t st) {
-    using RL = RowLayout<T>;
-    auto kern = quantize_rows_tma_kernel<T, BITS, PACK, CONV, BLOCKWISE, DYN>;
-    const int smem = kStages * RL::kTileBytes + 1024;
-    if (int e = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return e;
-    const int64_t n_tiles = (n_rows + kTileRows - 1) / kTileRows;
-    // DYN: one CTA per tile; resident CTAs steal the not-yet-launched ones (cluster launch control)
-    const unsigned grid = DYN ? (unsigned)n_tiles : (unsigned)grid_for_tiles(n_tiles);
-    cudaError_t e = launch_pdl(kern, dim3(grid), dim3(kTmaThreads), (size_t)smem, st, tmap, n_rows, log2_of(lanes_per_block), q, scale, zp,
-                               ws, nparts);
-    return cuda_status(e != cudaSuccess ? e : cudaGetLastError());
-}
-
-template <typename T, int BITS, bool PACK, int CONV, bool BLOCKWISE>
+template <typename T, int BITS, bool PACK>
 static int launch_rows_tma(const T* x, int64_t n_rows, int lanes_per_block, uint8_t* q, float* scale, float* zp,
-                           const float* ws, int nparts, cudaStream_t st) {
+                           cudaStream_t st) {
     using RL = RowLayout<T>;
     CUtensorMap tmap;
     int rc = make_tensor_map_2d(&tmap, TmaType<T>::v, sizeof(T), x, kRowElems, (uint64_t)n_rows, RL::kRowBytes,
                                 kRowElems, kTileRows,
                                 sizeof(T) == 4 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
     if (rc) return rc;
-    if (use_clc())
-        return launch_rows_tma_impl<T, BITS, PACK, CONV, BLOCKWISE, true>(tmap, n_rows, lanes_per_block, q, scale, zp, ws, nparts, st);
-    return launch_rows_tma_impl<T, BITS, PACK, CONV, BLOCKWISE, false>(tmap, n_rows, lanes_per_block, q, scale, zp, ws, nparts, st);
-}
-
-// SMs of the current device (the single-launch kernels put one CTA on each and synchronise them with
-// a grid barrier, so the grid must never exceed what is really there); cached per device.
-static int sm_count() {
-    static int cached[64] = {0};
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return kNumSMs;
-    if (cached[dev] == 0) {
-        int n = 0;
-        if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = kNumSMs;
-        cached[dev] = n < kNumSMs ? n : kNumSMs;          // the workspace partial slots are sized for kNumSMs
-    }
-    return cached[dev];
-}
-
-static bool use_fused_tensor() {
-    static const bool v = []() {
-        const char* e = getenv("QUANTA_B200_TWO_PASS");          // escape hatch: separate reduce + quantize launches
-        return !(e && e[0] == '1');
-    }();
-    return v;
+    auto kern = quantize_rows_tma_kernel<T, BITS, PACK>;
+    const int smem = kStages * RL::kTileBytes + 1024;
+    if (int e = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return e;
+    const int64_t n_tiles = (n_rows + kTileRows - 1) / kTileRows;
+    cudaError_t e = launch_pdl(kern, dim3((unsigned)n_tiles), dim3(kTmaThreads), (size_t)smem, st, tmap, n_rows,
+                               log2_of(lanes_per_block), q, scale, zp);
+    return cuda_status(e != cudaSuccess ? e : cudaGetLastError());
 }
 
 // One cooperative launch: a CTA per SM (or per tile when there are fewer tiles).
@@ -1620,13 +1425,12 @@ static int launch_tensor_fused(const T* x, int64_t n, int64_t n_rows, uint8_t* q
     int nslots = (224 * 1024) / kTileBytes;                      // 14 x 16 KB (+1 KB alignment) of the 227 KB an SM offers
     if (nslots > kFMaxSlots) nslots = kFMaxSlots;
     int ring_min = (128 * 1024) / kTileBytes;                    // 128 KB in flight per SM (a stage is held until its loads have returned)
-    { const int v = env_int("QUANTA_B200_FUSED_RING", 0); if (v >= kFGroups && v < nslots) ring_min = v; }
     ring_min = (ring_min + kFGroups - 1) / kFGroups * kFGroups;
     const int smem = nslots * kTileBytes + 1024;
     if (int e = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return e;
     const int64_t n_tiles = (n_rows + kFRows - 1) / kFRows;
     cudaLaunchConfig_t cfg = {};
-    const int sms = sm_count();
+    const int sms = device_sm_count();
     cfg.gridDim = dim3((unsigned)(n_tiles < sms ? n_tiles : sms));
     cfg.blockDim = dim3(kFThreads);
     cfg.dynamicSmemBytes = smem;
@@ -1636,7 +1440,6 @@ static int launch_tensor_fused(const T* x, int64_t n, int64_t n_rows, uint8_t* q
     attr[0].val.cooperative = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (env_int("QUANTA_B200_FUSED_COOP", 1) == 0) cfg.numAttrs = 0;
     return cuda_status(cudaLaunchKernelEx(&cfg, kern, tmap, x, n, n_rows, nslots, ring_min, q, scale, zp, ws));
 }
 
@@ -1650,7 +1453,7 @@ static int launch_dim0_fused(const T* x, int64_t rows, int64_t cols, uint8_t* q,
                              cudaStream_t st) {
     using RL = RowLayout<T>;
     constexpr int kTileBytes = kFRows * RL::kRowBytes;
-    if (cols % kRowElems != 0 || !aligned16(x) || !aligned16(q) || !use_fused_tensor()) return -1;
+    if (cols % kRowElems != 0 || !aligned16(x) || !aligned16(q)) return -1;
     // the second pass lives on L2 hits: beyond ~100 MB the re-read comes from HBM anyway and the
     // multi-launch path (more CTAs in flight) measured faster
     if ((double)rows * (double)cols * sizeof(T) > 100e6) return -1;
@@ -1659,7 +1462,7 @@ static int launch_dim0_fused(const T* x, int64_t rows, int64_t cols, uint8_t* q,
     if (tps * n_strips > (int64_t)1 << 30) return -1;
     geo.tps = (int)tps;
     geo.n_tiles = (int)(tps * n_strips);
-    const int sms = sm_count();
+    const int sms = device_sm_count();
     const int G = geo.n_tiles < sms ? geo.n_tiles : sms;
     const int per_cta = (geo.n_tiles + G - 1) / G;
     geo.max_strips = (per_cta + geo.tps - 1) / geo.tps + 1;
@@ -1686,7 +1489,6 @@ static int launch_dim0_fused(const T* x, int64_t rows, int64_t cols, uint8_t* q,
     attr[0].val.cooperative = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (env_int("QUANTA_B200_FUSED_COOP", 1) == 0) cfg.numAttrs = 0;
     return cuda_status(cudaLaunchKernelEx(&cfg, kern, tmap, rows, cols, geo, nslots, ring_min, q, scale, zp, ws));
 }
 
@@ -1697,32 +1499,22 @@ static int quantize_reduced(const T* x, int64_t rows, int64_t cols, int mode, ui
                             float* ws, cudaStream_t st) {
     const int64_t n = rows * cols;
     if (mode == QUANTA_MODE_TENSOR) {
-        float* pmin = ws + kWsHeaderFloats + 64;
-        float* pmax = pmin + kMaxPartialCtas;
-        int64_t want = (n + 256 * 16 - 1) / (256 * 16);
-        const int cap = kNumSMs * 4;                       // 4 resident CTAs of 256 threads per SM
-        int g = (int)(want < 1 ? 1 : (want > cap ? cap : want));
-        int64_t n_rows = aligned16(x) && aligned16(q) ? n / kRowElems : 0;
-        if (n_rows > 0 && use_fused_tensor()) {
+        const int64_t n_rows = aligned16(x) && aligned16(q) ? n / kRowElems : 0;
+        int64_t start = 0;
+        if (n_rows > 0) {
             int rc = launch_tensor_fused<T, BITS, PACK, CONV>(x, n, n_rows, q, scale, zp, ws, st);
             if (rc) return rc;
-            const int64_t start = n_rows * kRowElems;
-            if (start < n) {
-                int64_t pairs = (n - start + 1) / 2;
-                launch_pdl(quantize_generic_kernel<T, BITS, PACK, CONV>, dim3((unsigned)((pairs + 255) / 256)), dim3(256), 0, st, 
-                    x, start, n, 1, q, scale, zp, ws);
-            }
-            return cuda_status(cudaGetLastError());
-        }
-        launch_pdl(minmax_tensor_partial_kernel<T>, g, dim3(256), 0, st, x, n, pmin, pmax);
-        if (n_rows > 0) {
-            // the streaming kernel finalizes the reduction itself and publishes scale / zp
-            int rc = launch_rows_tma<T, BITS, PACK, CONV, false>(x, n_rows, 1, q, scale, zp, ws, g, st);
-            if (rc) return rc;
+            start = n_rows * kRowElems;
         } else {
+            // unaligned pointers (or fewer than kRowElems elements): partial min/max, finalize, generic quantize
+            float* pmin = ws + kWsHeaderFloats + 64;
+            float* pmax = pmin + kMaxPartialCtas;
+            int64_t want = (n + 256 * 16 - 1) / (256 * 16);
+            const int cap = kNumSMs * 4;                       // 4 resident CTAs of 256 threads per SM
+            int g = (int)(want < 1 ? 1 : (want > cap ? cap : want));
+            launch_pdl(minmax_tensor_partial_kernel<T>, g, dim3(256), 0, st, x, n, pmin, pmax);
             launch_pdl(minmax_tensor_finalize_kernel<CONV>, dim3(1), dim3(256), 0, st, pmin, pmax, g, BITS, scale, zp, ws);
         }
-        const int64_t start = n_rows * kRowElems;
         if (start < n) {
             int64_t pairs = (n - start + 1) / 2;
             launch_pdl(quantize_generic_kernel<T, BITS, PACK, CONV>, dim3((unsigned)((pairs + 255) / 256)), dim3(256), 0, st, 
@@ -1777,8 +1569,7 @@ static int quantize_affine_t(const T* x, int64_t rows, int64_t cols, int mode, i
     if (mode == QUANTA_MODE_BLOCK) {
         const int64_t nblocks = n / block;
         if (block % kRowElems == 0 && is_pow2(block / kRowElems) && block <= 1024 && aligned16(x) && aligned16(q))
-            return launch_rows_tma<T, BITS, PACK, kConvA, true>(x, n / kRowElems, (int)(block / kRowElems), q, scale, zp,
-                                                                ws, 0, st);
+            return launch_rows_tma<T, BITS, PACK>(x, n / kRowElems, (int)(block / kRowElems), q, scale, zp, st);
         if (PACK && (block & 1)) return QUANTA_EUNSUPPORTED;
         launch_pdl(quantize_block_generic_kernel<T, BITS, PACK>, dim3((unsigned)((nblocks + 7) / 8)), dim3(256), 0, st, x, nblocks, block, q,
                                                                                                   scale, zp);

@@ -2,7 +2,6 @@
 the composition the reference's layers imply: F.linear(x, dequantize(q).to(x.dtype))
 evaluated in float64 on the CPU (oracle.linear_dequant).  Tolerance (north_star):
 1e-2 relative in bf16 — measured as max|y - ref| / max|ref|."""
-import os
 
 import numpy as np
 import pytest
@@ -49,7 +48,7 @@ def rel_err(y, ref):
 @pytest.mark.parametrize("bits", [4, 8])
 @pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float16])
 @pytest.mark.parametrize("shape", [(128, 64, 1), (128, 256, 16), (256, 512, 5), (384, 1024, 33), (1024, 4096, 64),
-                                   (200, 320, 7), (512, 2048, 256), (256, 1024, 300)])
+                                   (200, 320, 7), (512, 2048, 256), (256, 1024, 300), (1004, 512, 48)])
 def test_gemm_matches_composition_oracle(bits, dtype, shape):
     from quanta_b200.nn import linear_wna16
     N, K, M = shape
@@ -170,46 +169,6 @@ def test_gemm_right_behind_the_kernel_that_wrote_its_weights(bits):
         torch.cuda.synchronize()
         bad += 0 if torch.equal(y, want[0]) else 1
     assert bad == 0
-
-
-def test_cta_pair_multicast_mode():
-    """QUANTA_B200_GEMM_PAIR=1: clusters of two CTAs on adjacent feature tiles, activation tiles multicast into both
-    (csrc/gemm.cu, CG = 2).  Off by default (no faster), so it runs here in a child process with the switch set: same
-    results as the default kernel (to one output ulp) on whole tiles, split tiles, ragged N (odd tile count), M > 256."""
-    import subprocess, sys, textwrap
-    code = textwrap.dedent("""
-        import os, sys, torch
-        sys.path.insert(0, os.getcwd())
-        import quanta_b200 as Q
-        from quanta_b200.nn import linear_wna16
-        out = {}
-        for (N, K, M, bits) in ((512, 2048, 128, 4), (384, 4096, 256, 8), (1000, 1024, 96, 4), (256, 8192, 300, 4), (2048, 512, 64, 8)):
-            g = torch.Generator().manual_seed(N + K + M)
-            w = (torch.randn(N, K, generator=g) * 0.02).cuda()
-            x = torch.randn(M, K, generator=g).to(torch.bfloat16).cuda()
-            b = (torch.randn(N, generator=g) * 0.1).to(torch.bfloat16).cuda()
-            q, s, z = Q.quantize_4bit(w, blocksize=64, packed=True) if bits == 4 else Q.quantize_8bit(w, blocksize=64)
-            y = linear_wna16(x, q, s, z, b, bits=bits, blocksize=64, out_features=N)
-            for _ in range(3):
-                assert torch.equal(linear_wna16(x, q, s, z, b, bits=bits, blocksize=64, out_features=N), y)
-            out[(N, K, M, bits)] = y.float().cpu()
-        torch.save(out, sys.argv[1])
-    """)
-    import tempfile
-    res = {}
-    with tempfile.TemporaryDirectory() as td:
-        for mode in ("0", "1"):
-            path = os.path.join(td, f"y{mode}.pt")
-            env = dict(os.environ, QUANTA_B200_GEMM_PAIR=mode)
-            r = subprocess.run([sys.executable, "-c", code, path], env=env, cwd=os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
-                               capture_output=True, text=True, timeout=300)
-            assert r.returncode == 0, r.stderr[-2000:]
-            res[mode] = torch.load(path)
-    for key, y0 in res["0"].items():
-        y1 = res["1"][key]
-        # the pair schedule cuts K at other places than the single-CTA one: same products, another fp32 summation order
-        err = float((y0 - y1).abs().max() / y0.abs().max())
-        assert err < 8e-3, f"pair mode differs for {key}: rel {err:.3e}"
 
 
 def test_gemm_repeated_calls_leave_workspace_clean():

@@ -1,7 +1,7 @@
 #!/bin/bash
 # tools/build_variant.sh <tag> [extra nvcc flags for gemm_small.cu ...]
 # Links quanta_b200/csrc/build/variants/lib<tag>.so from the regular objects plus a gemm_small.cu compiled with the
-# given flags (-DQUANTA_SMALL_TRACE: timeline stamps, -DQUANTA_SMALL_DBG: experiment switches).  For tools/ab_small.sh
+# given flags (-DQUANTA_SMALL_TRACE: timeline stamps).  For tools/ab_small.sh
 # and tools/trace_small.py; the variants are git-ignored and travel with the gpurun snapshot.
 set -e
 cd "$(dirname "$0")/../quanta_b200/csrc"
