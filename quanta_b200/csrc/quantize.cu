@@ -432,10 +432,17 @@ struct RowsMulti {
     __device__ __forceinline__ float* zp(int ti) const { return a.zp[ti]; }
 };
 
+// How a stream launch orders itself against its neighbours on the stream (programmatic dependent launch; the
+// argument is in common.cuh, next to pdl_wait).  kWaitFirst: wait for the previous kernel before the first global
+// access.  Without it the launch was released early by the previous multi-tensor launch of the same call, loads at
+// once and waits for that launch before it exits.  kReleaseNext: the next launch is the next multi-tensor launch of
+// the same call; let it start as soon as every CTA of this one has started (or been taken over) and is past its wait.
+constexpr int kWaitFirst = 1, kReleaseNext = 2;
+
 // Blockwise (convention A) row stream, one CTA per tile of the launch: resident CTAs steal the
 // not-yet-launched ones (cluster launch control).
 template <typename T, int BITS, bool PACK, typename Src>
-__device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_lanes_per_block) {
+__device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_lanes_per_block, int pdl) {
     using RL = RowLayout<T>;
     extern __shared__ uint8_t smem_raw[];
     __shared__ uint64_t full_bar[kStages], empty_bar[kStages], clc_bar;
@@ -454,13 +461,16 @@ __device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_la
         fence_barrier_init();
     }
     __syncthreads();
-    pdl_wait();                                            // the set-up above may overlap the previous kernel's tail
+    if (pdl & kWaitFirst) pdl_wait();                      // the set-up above may overlap the previous kernel's tail
+    if (pdl & kReleaseNext) asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
 
     if (warp == kConsumerWarps) {
         // ===== producer warp: one lane streams tiles into the ring =====
         if (lane == 0) {
             if (!Src::kMulti) prefetch_tensormap(src.map(0));
-            const uint64_t policy = policy_evict_first();
+            // evict-normal, not evict-first, although every tile is read once: measured 8 % faster on the
+            // bench step (profiles/INDEX.md, r03)
+            const uint64_t policy = policy_evict_normal();
             int cta = blockIdx.x;          // this CTA's own tile first, then stolen ones
             uint32_t clc_phase = 0;
             for (int i = 0;; ++i) {
@@ -482,6 +492,7 @@ __device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_la
                 cta = clc_read(smem_u32(&clc_resp));
             }
         }
+        if (!(pdl & kWaitFirst)) pdl_wait();               // our completion implies the previous launch's
         return;
     }
 
@@ -576,19 +587,20 @@ __device__ __forceinline__ void quantize_rows_stream(const Src& src, int log2_la
             }
         }
     }
+    if (!(pdl & kWaitFirst)) pdl_wait();
 }
 
 template <typename T, int BITS, bool PACK>
 __global__ void __launch_bounds__(kTmaThreads, 2)
 quantize_rows_tma_kernel(const __grid_constant__ CUtensorMap tmap, int64_t n_rows, int log2_lanes_per_block,
                          uint8_t* __restrict__ q_out, float* __restrict__ scale_out, float* __restrict__ zp_out) {
-    quantize_rows_stream<T, BITS, PACK>(RowsOne{&tmap, n_rows, q_out, scale_out, zp_out}, log2_lanes_per_block);
+    quantize_rows_stream<T, BITS, PACK>(RowsOne{&tmap, n_rows, q_out, scale_out, zp_out}, log2_lanes_per_block, kWaitFirst);
 }
 
 template <typename T, int BITS, bool PACK>
 __global__ void __launch_bounds__(kTmaThreads, 2)
-quantize_rows_tma_multi_kernel(const __grid_constant__ MultiArgs a, int log2_lanes_per_block) {
-    quantize_rows_stream<T, BITS, PACK>(RowsMulti{a}, log2_lanes_per_block);
+quantize_rows_tma_multi_kernel(const __grid_constant__ MultiArgs a, int log2_lanes_per_block, int pdl) {
+    quantize_rows_stream<T, BITS, PACK>(RowsMulti{a}, log2_lanes_per_block, pdl);
 }
 
 // --------------------------------------------------------------------------
@@ -1599,7 +1611,9 @@ static int backend_quantize_t(const T* x, int64_t rows, int64_t cols, int per_ch
 }
 
 // Blockwise batch: tensors that qualify for the TMA stream go through the multi-tensor kernel in
-// groups of kMultiMax; anything else falls back to a per-tensor launch.
+// groups of kMultiMax; anything else falls back to a per-tensor launch.  Consecutive multi-tensor
+// launches overlap: each releases the next early (kReleaseNext), which then waits before it exits
+// instead of before it starts; a per-tensor launch in between, and the end of the call, break the chain.
 template <typename T, int BITS, bool PACK>
 static int quantize_block_batch_t(const void* const* xs, const int64_t* numels, int count, int64_t block,
                                   uint8_t* const* qs, float* const* scales, float* const* zps, cudaStream_t st) {
@@ -1611,43 +1625,57 @@ static int quantize_block_batch_t(const void* const* xs, const int64_t* numels, 
     MultiArgs args;
     args.count = 0;
     args.tile_base[0] = 0;
-    auto flush = [&]() -> int {
+    bool released = false;                 // the previous launch on `st` is a multi-tensor launch that released us
+    auto flush = [&](bool release_next) -> int {
         if (args.count == 0) return QUANTA_OK;
+        const int pdl = (released ? 0 : kWaitFirst) | (release_next ? kReleaseNext : 0);
         cudaError_t le = launch_pdl(kern, dim3((unsigned)args.tile_base[args.count]), dim3(kTmaThreads), (size_t)smem, st, args,
-                                    log2_of(block / kRowElems));
+                                    log2_of(block / kRowElems), pdl);
         if (le != cudaSuccess) return (int)le;
+        released = release_next;
         args.count = 0;
         args.tile_base[0] = 0;
         return cuda_status(cudaGetLastError());
     };
+    // A launch that released the next one must be followed by it: otherwise the next programmatic launch on the
+    // stream could start before the released launch completes.  So an input error after a release still launches the
+    // pending group (which waits for its predecessor before it exits) before it is returned.  Only a failing launch
+    // can leave a released launch without its successor; the call returns that launch error.
+    auto fail = [&](int rc) -> int {
+        if (released) flush(false);
+        return rc;
+    };
     for (int i = 0; i < count; ++i) {
         const T* x = static_cast<const T*>(xs[i]);
         const int64_t n = numels[i];
-        if (n <= 0 || n % block != 0) return QUANTA_EINVAL;
+        if (n <= 0 || n % block != 0) return fail(QUANTA_EINVAL);
         const int64_t n_rows = n / kRowElems;
         const int64_t tiles = (n_rows + kTileRows - 1) / kTileRows;
         if (!shape_ok || !aligned16(x) || !aligned16(qs[i]) || tiles > (int64_t)1 << 24) {
-            int rc = flush();
+            int rc = flush(false);
             if (rc) return rc;
             rc = quantize_affine_t<T, BITS, PACK>(x, 1, n, QUANTA_MODE_BLOCK, block, qs[i], scales[i], zps[i], nullptr, st);
             if (rc) return rc;
             continue;
         }
+        // encoded before a flush that releases the next launch, so that a releasing flush always has a group to follow it
+        CUtensorMap map;
+        int rc = make_tensor_map_2d(&map, TmaType<T>::v, sizeof(T), x, kRowElems, (uint64_t)n_rows, RL::kRowBytes,
+                                    kRowElems, kTileRows,
+                                    sizeof(T) == 4 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
+        if (rc) return fail(rc);
         if (args.count == kMultiMax || (int64_t)args.tile_base[args.count] + tiles > (int64_t)1 << 30) {
-            int rc = flush();
+            rc = flush(true);
             if (rc) return rc;
         }
         const int k = args.count;
-        int rc = make_tensor_map_2d(&args.maps[k], TmaType<T>::v, sizeof(T), x, kRowElems, (uint64_t)n_rows, RL::kRowBytes,
-                                    kRowElems, kTileRows,
-                                    sizeof(T) == 4 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
-        if (rc) return rc;
+        args.maps[k] = map;
         args.n_rows[k] = n_rows;
         args.q[k] = qs[i]; args.scale[k] = scales[i]; args.zp[k] = zps[i];
         args.tile_base[k + 1] = args.tile_base[k] + (int)tiles;
         args.count = k + 1;
     }
-    return flush();
+    return flush(false);
 }
 
 size_t quantize_workspace_bytes(int64_t cols) {
