@@ -298,6 +298,27 @@ QUANTA_API int quanta_gemm_nf4a16(const void* x, int act_dtype, const uint8_t* w
                        int64_t block, const void* bias, void* y, int64_t M, int64_t N, int64_t K,
                        void* workspace, size_t workspace_bytes, void* stream);
 
+/* Input gradient of quanta_gemm_wna16 (the backward of Linear4bit /
+ * Linear8bitLt for a frozen quantized weight):
+ *     dx[M,K] = dy[M,N] . dequant(Wq)[N,K]
+ * with wq / scale / zp / block exactly as passed to the forward; the
+ * weights are dequantized to bit-for-bit the 16-bit values the forward
+ * multiplies with.  dy, dx are `act_dtype` (F16 or BF16), fp32 accumulation.
+ * dy rows have a pitch of round_up(N, 8) elements (16-byte aligned rows for
+ * TMA); columns N .. pitch-1 are never read.  dx is [M, K] contiguous.
+ * workspace: quanta_workspace_bytes(QUANTA_OP_GEMM, M, K), the same
+ * zero-initialised buffer as the forward's (the counters are left zero).  */
+QUANTA_API int quanta_gemm_wna16_dgrad(const void* dy, int act_dtype, const uint8_t* wq, int bits,
+                            const float* scale, const float* zp, int64_t block, void* dx,
+                            int64_t M, int64_t N, int64_t K,
+                            void* workspace, size_t workspace_bytes, void* stream);
+
+/* The same for NF4 weights (quanta_gemm_nf4a16):
+ * dx = dy . (level[code] * absmax)[N,K].                                    */
+QUANTA_API int quanta_gemm_nf4a16_dgrad(const void* dy, int act_dtype, const uint8_t* wq, const float* absmax,
+                             int64_t block, void* dx, int64_t M, int64_t N, int64_t K,
+                             void* workspace, size_t workspace_bytes, void* stream);
+
 /* LLM.int8()-style outlier-split matmul for Linear8bitLt.threshold
  * (nn/linear.py:20,25; unused by the reference — semantics defined by this
  * repository, see oracle/oracle_np.py:int8_outlier_matmul).

@@ -53,6 +53,8 @@ SIGNATURES = {
                                               _sz, _vp, _int, _int, _vp, _vp]),
     "quanta_peer_barrier": (_int, [_vp, _int, _int, _vp, _vp]),
     "quanta_gemm_nf4a16": (_int, [_vp, _int, _vp, _vp, _i64, _vp, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
+    "quanta_gemm_wna16_dgrad": (_int, [_vp, _int, _vp, _int, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
+    "quanta_gemm_nf4a16_dgrad": (_int, [_vp, _int, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
     "quanta_int8_outlier_matmul": (_int, [_vp, _int, _vp, _vp, _f, _vp, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
 }
 

@@ -157,6 +157,118 @@ def linear_nf4a16(x, wq, absmax, bias=None, blocksize=64, out_features=None, in_
     return y.reshape(*x.shape[:-1], N)
 
 
+def _dgrad_args(dy, wq, bits, out_features, in_features, what):
+    """dy as the [M, round_up(N, 8)] matrix the dgrad entries read (zero columns past N), and (N, K)."""
+    _host.require_cuda(dy, "dy")
+    if dy.dtype not in (torch.float16, torch.bfloat16):
+        raise TypeError("dy must be float16 or bfloat16")
+    N = dy.shape[-1]
+    if out_features is not None and out_features != N:
+        raise ValueError(f"{what}: dy has {N} features, layer has {out_features} outputs")
+    if in_features is None:
+        if N == 0 or not isinstance(wq, torch.Tensor):
+            raise ValueError(f"{what}: in_features is required")
+        in_features = wq.numel() * 8 // bits // N
+    dy2 = dy.reshape(-1, N)
+    if N % 8:
+        dy2 = torch.nn.functional.pad(dy2, (0, 8 - N % 8))
+    if not dy2.is_contiguous():
+        dy2 = dy2.contiguous()
+    return dy2, N, in_features
+
+
+def linear_wna16_dgrad(dy, wq, scale, zp, bits=4, blocksize=64, out_features=None, in_features=None):
+    """dx = dy @ dequant(Wq): the input gradient of ``linear_wna16`` for a frozen weight, with the weights
+    dequantized to bit-for-bit the 16-bit values the forward multiplies with.
+
+    dy     [..., N]   float16 / bfloat16 (CUDA);  returns dx [..., K] in dy's dtype
+    wq, scale, zp, bits, blocksize as for ``linear_wna16``"""
+    if bits not in (4, 8):
+        raise ValueError("bits must be 4 or 8")
+    dy2, N, K = _dgrad_args(dy, wq, bits, out_features, in_features, "linear_wna16_dgrad")
+    _check_weight_args(dy, wq, (("scale", scale), ("zero_point", zp)), N, K, bits, blocksize, "linear_wna16_dgrad")
+    M = dy2.shape[0]
+    dev = dy.device
+    dx = torch.empty((M, K), dtype=dy.dtype, device=dev)
+    if M == 0 or N == 0:
+        return dx.zero_().reshape(*dy.shape[:-1], K)
+    with _host.device_guard(dev):
+        ws = _host.gemm_workspace(dev, _host.workspace_bytes(_lib.OP_GEMM, M, K))
+        st = _lib.lib().quanta_gemm_wna16_dgrad(dy2.data_ptr(), _host.dtype_code(dy2), wq.data_ptr(), bits, scale.data_ptr(),
+                                                zp.data_ptr(), blocksize, dx.data_ptr(), M, N, K, ws.data_ptr(), ws.numel(),
+                                                _host.stream_ptr(dev))
+    _lib.check(st, "quanta_gemm_wna16_dgrad")
+    return dx.reshape(*dy.shape[:-1], K)
+
+
+def linear_nf4a16_dgrad(dy, wq, absmax, blocksize=64, out_features=None, in_features=None):
+    """dx = dy @ (nf4_level[Wq] * absmax): the input gradient of ``linear_nf4a16`` for a frozen weight."""
+    dy2, N, K = _dgrad_args(dy, wq, 4, out_features, in_features, "linear_nf4a16_dgrad")
+    _check_weight_args(dy, wq, (("absmax", absmax),), N, K, 4, blocksize, "linear_nf4a16_dgrad")
+    M = dy2.shape[0]
+    dev = dy.device
+    dx = torch.empty((M, K), dtype=dy.dtype, device=dev)
+    if M == 0 or N == 0:
+        return dx.zero_().reshape(*dy.shape[:-1], K)
+    with _host.device_guard(dev):
+        ws = _host.gemm_workspace(dev, _host.workspace_bytes(_lib.OP_GEMM, M, K))
+        st = _lib.lib().quanta_gemm_nf4a16_dgrad(dy2.data_ptr(), _host.dtype_code(dy2), wq.data_ptr(), absmax.data_ptr(),
+                                                 blocksize, dx.data_ptr(), M, N, K, ws.data_ptr(), ws.numel(),
+                                                 _host.stream_ptr(dev))
+    _lib.check(st, "quanta_gemm_nf4a16_dgrad")
+    return dx.reshape(*dy.shape[:-1], K)
+
+
+class LinearWNA16Function(torch.autograd.Function):
+    """``linear_wna16`` with a backward for x and bias; the quantized weight is frozen and gets no gradient.
+
+    ``bias`` is the parameter the gradient goes to; ``bias_k`` is the same values as the kernel reads them
+    (x's dtype, contiguous).  A double backward is not supported."""
+
+    @staticmethod
+    def forward(ctx, x, bias, bias_k, wq, scale, zp, bits, blocksize, out_features, in_features):
+        ctx.save_for_backward(wq, scale, zp)
+        ctx.meta = (bits, blocksize, out_features, in_features)
+        ctx.bias_dtype = bias.dtype if bias is not None else None
+        return linear_wna16(x, wq, scale, zp, bias_k, bits=bits, blocksize=blocksize, out_features=out_features,
+                            in_features=in_features)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dy):
+        wq, scale, zp = ctx.saved_tensors
+        bits, blocksize, N, K = ctx.meta
+        dx = db = None
+        if ctx.needs_input_grad[0]:
+            dx = linear_wna16_dgrad(dy, wq, scale, zp, bits=bits, blocksize=blocksize, out_features=N, in_features=K)
+        if ctx.needs_input_grad[1]:
+            db = dy.reshape(-1, N).sum(0, dtype=torch.float32).to(ctx.bias_dtype)
+        return dx, db, None, None, None, None, None, None, None, None
+
+
+class LinearNF4A16Function(torch.autograd.Function):
+    """``linear_nf4a16`` with a backward for x and bias (see ``LinearWNA16Function``)."""
+
+    @staticmethod
+    def forward(ctx, x, bias, bias_k, wq, absmax, blocksize, out_features, in_features):
+        ctx.save_for_backward(wq, absmax)
+        ctx.meta = (blocksize, out_features, in_features)
+        ctx.bias_dtype = bias.dtype if bias is not None else None
+        return linear_nf4a16(x, wq, absmax, bias_k, blocksize=blocksize, out_features=out_features, in_features=in_features)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dy):
+        wq, absmax = ctx.saved_tensors
+        blocksize, N, K = ctx.meta
+        dx = db = None
+        if ctx.needs_input_grad[0]:
+            dx = linear_nf4a16_dgrad(dy, wq, absmax, blocksize=blocksize, out_features=N, in_features=K)
+        if ctx.needs_input_grad[1]:
+            db = dy.reshape(-1, N).sum(0, dtype=torch.float32).to(ctx.bias_dtype)
+        return dx, db, None, None, None, None, None, None
+
+
 def rowwise_quantize_sym(weight):
     """Static int8 weight codes for the outlier-split matmul: convention-B
     symmetric 8-bit with one multiplier per OUTPUT row, i.e.

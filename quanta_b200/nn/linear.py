@@ -11,6 +11,14 @@ along in_features) and ``forward`` is the fused dequantize-then-matmul kernel:
 Parity: defined by that composition (SURVEY §8(c)); tolerance 1e-2 relative in
 bf16/fp16.  ``Linear4bit`` supports ``quant_type="nf4"`` (the reference default: NF4 codebook,
 blockwise abs_max) and ``quant_type="linear"`` (blockwise affine).
+
+Backward: the quantized weight is frozen (its codes are buffers).  When autograd is recording and x or
+the bias requires a gradient, ``Linear4bit`` and ``Linear8bitLt(outlier_split=False)`` run through an
+autograd Function whose backward gives ``x.grad = dy @ W`` (the fused dequantize-transposed GEMM,
+with bit-for-bit the weights of the forward) and ``bias.grad = dy.sum(0)`` (fp32 accumulation).  The
+forward launches the same kernel with the same arguments either way.  Not differentiable: the
+outlier split (``outlier_split=True``), the tensor-parallel layers, the weight itself, and a double
+backward.
 """
 from __future__ import annotations
 
@@ -20,7 +28,8 @@ import torch
 import torch.nn as nn
 
 from ..functional.quantization import quantize_4bit, quantize_8bit, dequantize_4bit, dequantize_8bit
-from .functional import linear_wna16, linear_nf4a16, int8_outlier_matmul, rowwise_quantize_sym
+from .functional import (linear_wna16, linear_nf4a16, int8_outlier_matmul, rowwise_quantize_sym, LinearWNA16Function,
+                         LinearNF4A16Function)
 
 
 _QUANT_BUFFERS = ("qweight", "scale", "zero_point", "qweight_rowwise", "row_scale")
@@ -150,9 +159,18 @@ class _QuantLinearBase(nn.Module):
                 raise RuntimeError("quanta_b200 layers run on CUDA only: move the module to a GPU first")
             self.quantize_()
         xin = x if x.dtype == compute_dtype else x.to(compute_dtype)
-        y = linear_wna16(xin, self.qweight, self.scale, self.zero_point, self._bias_as(compute_dtype, x.device), bits=self.bits,
-                         blocksize=self.blocksize, out_features=self.out_features, in_features=self.in_features)
+        if self._records_grad(xin):
+            y = LinearWNA16Function.apply(xin, self.bias, self._bias_as(compute_dtype, x.device), self.qweight, self.scale,
+                                          self.zero_point, self.bits, self.blocksize, self.out_features, self.in_features)
+        else:
+            y = linear_wna16(xin, self.qweight, self.scale, self.zero_point, self._bias_as(compute_dtype, x.device),
+                             bits=self.bits, blocksize=self.blocksize, out_features=self.out_features,
+                             in_features=self.in_features)
         return y if y.dtype == x.dtype or not x.is_floating_point() else y.to(x.dtype)
+
+    def _records_grad(self, x):
+        """Whether autograd needs this call: grad mode on and x or the bias requires a gradient."""
+        return torch.is_grad_enabled() and (x.requires_grad or (self.bias is not None and self.bias.requires_grad))
 
 
 class Linear8bitLt(_QuantLinearBase):
@@ -162,7 +180,10 @@ class Linear8bitLt(_QuantLinearBase):
     ``outlier_split=True``: the LLM.int8() decomposition the reference's
     ``threshold`` argument points at (row G3) — row-wise symmetric int8 weight
     codes, int8 x int8 tensor-core product for the regular feature columns and
-    a 16-bit product for the columns whose activations exceed ``threshold``."""
+    a 16-bit product for the columns whose activations exceed ``threshold``.
+
+    Differentiable in x and bias with ``outlier_split=False`` (module docstring); the outlier split
+    is inference-only."""
     bits = 8
 
     def __init__(self, in_features, out_features, bias=True, has_fp16_weights=False, threshold=6.0, blocksize=64,
@@ -206,7 +227,9 @@ class Linear4bit(_QuantLinearBase):
     """4-bit quantized linear layer (Quanta/nn/linear.py:48-83).
 
     ``quant_type="nf4"`` (the reference default): NF4 codebook with one abs_max per block of
-    ``blocksize`` input features; ``quant_type="linear"``: blockwise affine min-max (convention A)."""
+    ``blocksize`` input features; ``quant_type="linear"``: blockwise affine min-max (convention A).
+    Both are differentiable in x and bias (module docstring): the QLoRA setting of a frozen NF4 base
+    under trainable adapters gets the base's ``dy @ W`` term in ``x.grad``."""
     bits = 4
 
     def __init__(self, in_features, out_features, bias=True, compute_dtype=torch.float16, quant_type="nf4",
@@ -249,6 +272,10 @@ class Linear4bit(_QuantLinearBase):
                 raise RuntimeError("quanta_b200 layers run on CUDA only: move the module to a GPU first")
             self.quantize_()
         xin = x if x.dtype == self.compute_dtype else x.to(self.compute_dtype)
-        y = linear_nf4a16(xin, self.qweight, self.scale, self._bias_as(self.compute_dtype, x.device), blocksize=self.blocksize,
-                          out_features=self.out_features, in_features=self.in_features)
+        if self._records_grad(xin):
+            y = LinearNF4A16Function.apply(xin, self.bias, self._bias_as(self.compute_dtype, x.device), self.qweight,
+                                           self.scale, self.blocksize, self.out_features, self.in_features)
+        else:
+            y = linear_nf4a16(xin, self.qweight, self.scale, self._bias_as(self.compute_dtype, x.device),
+                              blocksize=self.blocksize, out_features=self.out_features, in_features=self.in_features)
         return y if y.dtype == x.dtype or not x.is_floating_point() else y.to(x.dtype)
