@@ -64,7 +64,7 @@ gemm_wna16_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
     if (tid == 32 * kFirstEpiWarp) fin_tile = -1;       // before the CTA-wide barrier below
     if (BITS == 4 && p.nf4 && tid >= 32 * kFirstDqWarp && tid < 32 * kFirstDqWarp + 256) {
         const int b = tid - 32 * kFirstDqWarp;      // visible to the dequant warps after the CTA-wide barrier below
-        nf4_pairs[b] = AT::pack(kGemmNf4Levels[b & 15], kGemmNf4Levels[b >> 4]);
+        nf4_pairs[b] = AT::pack(kNf4Levels[b & 15], kNf4Levels[b >> 4]);
     }
 
     // Programmatic dependent launch: the next kernel on the stream may start its prologue while this grid is in

@@ -95,7 +95,7 @@ gemm_dgrad_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
     if (tid == 32 * kDgFirstEpiWarp) fin_tile = -1;
     if (BITS == 4 && p.nf4 && tid >= 32 * kDgFirstDqWarp && tid < 32 * kDgFirstDqWarp + 256) {
         const int b = tid - 32 * kDgFirstDqWarp;
-        nf4_pairs[b] = AT::pack(kGemmNf4Levels[b & 15], kGemmNf4Levels[b >> 4]);
+        nf4_pairs[b] = AT::pack(kNf4Levels[b & 15], kNf4Levels[b >> 4]);
     }
 
     // PDL as in the forward: release dependents at once; the weight stream (codes, scales) starts

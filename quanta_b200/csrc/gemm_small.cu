@@ -41,6 +41,7 @@
 // to the activation type first, like the reference's `.to(x.dtype)`); the difference is far inside
 // the 1e-2 tolerance of rows G1/G2.
 #include "common.cuh"
+#include "nf4_levels.cuh"
 
 #include <type_traits>
 
@@ -73,13 +74,6 @@ template <int BITS, bool NF4 = false> struct SmGeom {
     static constexpr uint32_t kStageBytes = kCodeBytes + (NF4 ? 1u : 2u) * kParamTile;   // codes | scales (NF4: abs_max) | zero-points
 };
 constexpr uint32_t kSmLutBytes = 256u * 128u;   // NF4: byte -> (level[lo nibble], level[hi nibble]) in the activation type, one copy per lane
-
-// NF4 levels (Quanta/functional/quantization.py:101-118; the same table as nf4.cu / gemm.cu)
-__constant__ float kSmNf4Levels[16] = {
-    -1.0f, -0.6961928009986877f, -0.5250730514526367f, -0.39491748809814453f, -0.28444138169288635f,
-    -0.18477343022823334f, -0.09105003625154495f, 0.0f, 0.07958029955625534f, 0.16093020141124725f,
-    0.24611230194568634f, 0.33791524171829224f, 0.44070982933044434f, 0.5626170039176941f,
-    0.7229568362236023f, 1.0f};
 
 // Timeline of one launch (-DQUANTA_SMALL_TRACE build only): per CTA 40 clock64 stamps relative to kernel entry, + globaltimer at
 // entry / exit in slots 38 / 39.  Read back with quanta_debug_small_trace().
@@ -590,7 +584,7 @@ gemm_small_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
     if (NF4) {
         for (int e = tid; e < 256 * 32; e += kSmConsThreads) {
             const int b = e >> 5;
-            const uint32_t pr = T::pack(kSmNf4Levels[b & 15], kSmNf4Levels[b >> 4]);
+            const uint32_t pr = T::pack(kNf4Levels[b & 15], kNf4Levels[b >> 4]);
             asm volatile("st.shared.b32 [%0], %1;" ::"r"(smem + p.lut_off + (uint32_t)e * 4u), "r"(pr) : "memory");
         }
         sm_cons_sync();

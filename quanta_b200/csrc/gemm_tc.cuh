@@ -3,6 +3,7 @@
 // same instructions, so the backward multiplies with bit-for-bit the weights the forward used.
 #pragma once
 #include "common.cuh"
+#include "nf4_levels.cuh"
 
 #include <cmath>
 
@@ -152,12 +153,6 @@ __device__ __forceinline__ void dequant_word8(uint32_t w, float s, float zc, uin
     out[0] = ActTraits<ACT>::pack(f[0], f[1]);
     out[1] = ActTraits<ACT>::pack(f[2], f[3]);
 }
-
-static __constant__ float kGemmNf4Levels[16] = {
-    -1.0f, -0.6961928009986877f, -0.5250730514526367f, -0.39491748809814453f,
-    -0.28444138169288635f, -0.18477343022823334f, -0.09105003625154495f, 0.0f,
-    0.07958029955625534f, 0.16093020141124725f, 0.24611230194568634f, 0.33791524171829224f,
-    0.44070982933044434f, 0.5626170039176941f, 0.7229568362236023f, 1.0f};
 
 constexpr int kMaxOut = 8;
 // NOUT = 1 for the plain GEMM (one map, compile-time loops), kMaxOut for the scatter entry

@@ -22,8 +22,7 @@ import torch
 
 from .. import _host, _lib
 
-_nf8_levels = {}
-_nf4_levels = {}
+_levels = {}          # (quant_type, str(device)) -> the codebook's levels as a float32 tensor on that device
 
 
 def _quantize_linear(tensor, bits, per_channel, blocksize, packed):
@@ -76,82 +75,27 @@ def _quantize_linear(tensor, bits, per_channel, blocksize, packed):
     return q, scale.reshape(pshape), zp.reshape(pshape)
 
 
+def _codebook_levels(quant_type, device):
+    import ctypes as C
+    key = (quant_type, str(device))
+    if key not in _levels:
+        count, entry = (16, "quanta_nf4_levels") if quant_type == "nf4" else (256, "quanta_nf8_levels")
+        buf = (C.c_float * count)()
+        _lib.check(getattr(_lib.lib(), entry)(buf), entry)
+        _levels[key] = torch.tensor(list(buf), dtype=torch.float32, device=device)
+    return _levels[key]
+
+
 def nf4_levels(device):
     """The 16 NF4 levels as a float32 tensor on ``device`` (second return value of the reference's
     ``quantize_4bit(..., quant_type="nf4")``, Quanta/functional/quantization.py:105-110)."""
-    import ctypes as C
-    key = str(device)
-    if key not in _nf4_levels:
-        buf = (C.c_float * 16)()
-        _lib.check(_lib.lib().quanta_nf4_levels(buf), "quanta_nf4_levels")
-        _nf4_levels[key] = torch.tensor(list(buf), dtype=torch.float32, device=device)
-    return _nf4_levels[key]
-
-
-def _quantize_nf4(tensor, blocksize, packed):
-    _host.require_cuda(tensor)
-    x = tensor.detach()
-    if not x.is_contiguous():
-        x = x.contiguous()
-    code = _host.dtype_code(x)
-    n = x.numel()
-    if n == 0:
-        raise RuntimeError("max(): cannot quantize an empty tensor")
-    dev = x.device
-    B = 0 if blocksize is None else int(blocksize)
-    if B and n % B:
-        raise ValueError(f"numel ({n}) must be a multiple of blocksize ({blocksize})")
-    if B and (B < 16 or B > 512 or (B & (B - 1))):
-        raise ValueError(f"NF4 blocksize must be 16 * 2^j <= 512 (got {blocksize}); the affine formats take any block size")
-    with _host.device_guard(dev):
-        q = torch.empty((n + 1) // 2 if packed else n, dtype=torch.uint8, device=dev)
-        absmax = torch.empty(n // B if B else 1, dtype=torch.float32, device=dev)
-        st = _lib.lib().quanta_quantize_nf4(x.data_ptr(), code, n, B, int(bool(packed)), q.data_ptr(),
-                                            absmax.data_ptr(), _host.stream_ptr(dev))
-    _lib.check(st, "quanta_quantize_nf4")
-    if not packed:
-        q = q.reshape(tensor.shape)
-    return q, nf4_levels(dev), (absmax if B else absmax.reshape(()))
-
-
-def _dequantize_nf4(q_tensor, absmax, blocksize, packed, shape, out_dtype):
-    _host.require_cuda(q_tensor, "q_tensor")
-    dev = q_tensor.device
-    q = q_tensor.detach()
-    if q.dtype != torch.uint8:
-        q = q.to(torch.uint8)
-    if not q.is_contiguous():
-        q = q.contiguous()
-    absmax = torch.as_tensor(absmax, dtype=torch.float32, device=dev).reshape(-1).contiguous()
-    out_shape = (torch.Size(shape) if shape is not None else torch.Size([q.numel() * 2])) if packed else q.shape
-    n = out_shape.numel()
-    if packed and q.numel() != (n + 1) // 2:
-        raise ValueError(f"packed codes hold {q.numel()} bytes, shape {tuple(out_shape)} needs {(n + 1) // 2}")
-    out = torch.empty(out_shape, dtype=out_dtype, device=dev)
-    if n == 0:
-        return out
-    B = 0 if blocksize is None else int(blocksize)
-    if B and (B < 16 or B > 512 or (B & (B - 1))):
-        raise ValueError(f"NF4 blocksize must be 16 * 2^j <= 512 (got {blocksize}); the affine formats take any block size")
-    if (B and absmax.numel() != n // B) or (not B and absmax.numel() != 1):
-        raise ValueError("absmax does not match blocksize")
-    with _host.device_guard(dev):
-        st = _lib.lib().quanta_dequantize_nf4(q.data_ptr(), int(bool(packed)), n, B, absmax.data_ptr(), out.data_ptr(),
-                                              _host._DTYPE[out_dtype], _host.stream_ptr(dev))
-    _lib.check(st, "quanta_dequantize_nf4")
-    return out
+    return _codebook_levels("nf4", device)
 
 
 def nf8_levels(device):
     """The 256 nf8 levels ``tanh(2 * linspace(-1, 1, 256))`` exactly as the reference's torch computes them
     (second return value of ``quantize_8bit(..., quant_type="nf8")``, Quanta/functional/quantization.py:174-175)."""
-    import ctypes as C
-    key = str(device)
-    if key not in _nf8_levels:
-        buf = (C.c_float * 256)()
-        _lib.check(_lib.lib().quanta_nf8_levels(buf), "quanta_nf8_levels")
-        _nf8_levels[key] = torch.tensor(list(buf), dtype=torch.float32, device=device)
-    return _nf8_levels[key]
+    return _codebook_levels("nf8", device)
 
 
 def _prep_input(tensor):
@@ -162,41 +106,84 @@ def _prep_input(tensor):
     return x, _host.dtype_code(x), x.numel(), x.device
 
 
-def _quantize_nf8(tensor, blocksize):
+def _prep_codes(q_tensor):
+    """The codes argument of a dequantize call as a contiguous uint8 CUDA tensor."""
+    _host.require_cuda(q_tensor, "q_tensor")
+    q = q_tensor.detach()
+    if q.dtype != torch.uint8:
+        q = q.to(torch.uint8)
+    if not q.is_contiguous():
+        q = q.contiguous()
+    return q
+
+
+def _out_shape(q, packed, shape):
+    """Shape of the dequantized output: the codes' shape, or for nibble-packed codes ``shape`` (default: two values per
+    byte), which must need exactly the bytes ``q`` holds."""
+    if not packed:
+        return q.shape
+    out_shape = torch.Size(shape) if shape is not None else torch.Size([q.numel() * 2])
+    n = out_shape.numel()
+    if q.numel() != (n + 1) // 2:
+        # a wrong ``shape`` would make the kernel read past the packed buffer
+        raise ValueError(f"packed codes hold {q.numel()} bytes, shape {tuple(out_shape)} needs {(n + 1) // 2}")
+    return out_shape
+
+
+def _check_nf4_blocksize(B, blocksize):
+    if B and (B < 16 or B > 512 or (B & (B - 1))):
+        raise ValueError(f"NF4 blocksize must be 16 * 2^j <= 512 (got {blocksize}); the affine formats take any block size")
+
+
+def _quantize_codebook(tensor, quant_type, blocksize, packed=False):
+    """NF4 / nf8: returns ``(codes, levels, abs_max)`` like the reference (:118, :183).  Only NF4 packs; nf8 leaves
+    an unsupported block size to the C entry."""
     x, code, n, dev = _prep_input(tensor)
     if n == 0:
         raise RuntimeError("max(): cannot quantize an empty tensor")
     B = 0 if blocksize is None else int(blocksize)
     if B and n % B:
         raise ValueError(f"numel ({n}) must be a multiple of blocksize ({blocksize})")
+    if quant_type == "nf4":
+        _check_nf4_blocksize(B, blocksize)
     with _host.device_guard(dev):
-        q = torch.empty(n, dtype=torch.uint8, device=dev)
+        q = torch.empty((n + 1) // 2 if packed else n, dtype=torch.uint8, device=dev)
         absmax = torch.empty(n // B if B else 1, dtype=torch.float32, device=dev)
-        st = _lib.lib().quanta_quantize_nf8(x.data_ptr(), code, n, B, q.data_ptr(), absmax.data_ptr(), _host.stream_ptr(dev))
-    _lib.check(st, "quanta_quantize_nf8")
-    return q.reshape(tensor.shape), nf8_levels(dev), (absmax if B else absmax.reshape(()))
+        if quant_type == "nf4":
+            st = _lib.lib().quanta_quantize_nf4(x.data_ptr(), code, n, B, int(bool(packed)), q.data_ptr(),
+                                                absmax.data_ptr(), _host.stream_ptr(dev))
+        else:
+            st = _lib.lib().quanta_quantize_nf8(x.data_ptr(), code, n, B, q.data_ptr(), absmax.data_ptr(),
+                                                _host.stream_ptr(dev))
+    _lib.check(st, f"quanta_quantize_{quant_type}")
+    if not packed:
+        q = q.reshape(tensor.shape)
+    return q, _codebook_levels(quant_type, dev), (absmax if B else absmax.reshape(()))
 
 
-def _dequantize_nf8(q_tensor, absmax, blocksize, out_dtype):
-    _host.require_cuda(q_tensor, "q_tensor")
-    dev = q_tensor.device
-    q = q_tensor.detach()
-    if q.dtype != torch.uint8:
-        q = q.to(torch.uint8)
-    if not q.is_contiguous():
-        q = q.contiguous()
+def _dequantize_codebook(q_tensor, absmax, quant_type, blocksize, packed, shape, out_dtype):
+    """``levels[q] * abs_max`` for NF4 (optionally nibble-packed) and nf8."""
+    q = _prep_codes(q_tensor)
+    dev = q.device
     absmax = torch.as_tensor(absmax, dtype=torch.float32, device=dev).reshape(-1).contiguous()
-    n = q.numel()
-    out = torch.empty(q.shape, dtype=out_dtype, device=dev)
+    out_shape = _out_shape(q, packed, shape)
+    n = out_shape.numel()
+    out = torch.empty(out_shape, dtype=out_dtype, device=dev)
     if n == 0:
         return out
     B = 0 if blocksize is None else int(blocksize)
+    if quant_type == "nf4":
+        _check_nf4_blocksize(B, blocksize)
     if (B and absmax.numel() != n // B) or (not B and absmax.numel() != 1):
         raise ValueError("absmax does not match blocksize")
     with _host.device_guard(dev):
-        st = _lib.lib().quanta_dequantize_nf8(q.data_ptr(), n, B, absmax.data_ptr(), out.data_ptr(),
-                                              _host._DTYPE[out_dtype], _host.stream_ptr(dev))
-    _lib.check(st, "quanta_dequantize_nf8")
+        if quant_type == "nf4":
+            st = _lib.lib().quanta_dequantize_nf4(q.data_ptr(), int(bool(packed)), n, B, absmax.data_ptr(),
+                                                  out.data_ptr(), _host._DTYPE[out_dtype], _host.stream_ptr(dev))
+        else:
+            st = _lib.lib().quanta_dequantize_nf8(q.data_ptr(), n, B, absmax.data_ptr(), out.data_ptr(),
+                                                  _host._DTYPE[out_dtype], _host.stream_ptr(dev))
+    _lib.check(st, f"quanta_dequantize_{quant_type}")
     return out
 
 
@@ -212,13 +199,8 @@ def _quantize_fp(tensor, bits):
 
 
 def _dequantize_fp(q_tensor, bias, bits, out_dtype):
-    _host.require_cuda(q_tensor, "q_tensor")
-    dev = q_tensor.device
-    q = q_tensor.detach()
-    if q.dtype != torch.uint8:
-        q = q.to(torch.uint8)
-    if not q.is_contiguous():
-        q = q.contiguous()
+    q = _prep_codes(q_tensor)
+    dev = q.device
     if float(bias) != int(bias):
         raise ValueError("the exponent bias must be an integer")
     out = torch.empty(q.shape, dtype=out_dtype, device=dev)
@@ -237,7 +219,7 @@ def quantize_4bit(tensor, quant_type="linear", per_channel=False, blocksize=None
         return _quantize_linear(tensor, 4, per_channel, blocksize, packed)
     if quant_type == "nf4":
         # returns (indices, nf4_levels, abs_max) like the reference (:118)
-        return _quantize_nf4(tensor, blocksize, packed)
+        return _quantize_codebook(tensor, "nf4", blocksize, packed)
     if quant_type == "fp4":
         return _quantize_fp(tensor, 4)
     raise ValueError(f"Unknown quantization type: {quant_type}")
@@ -250,7 +232,7 @@ def quantize_8bit(tensor, quant_type="linear", per_channel=False, blocksize=None
         return _quantize_linear(tensor, 8, per_channel, blocksize, False)
     if quant_type == "nf8":
         # returns (indices, nf8_levels, abs_max) like the reference (:183)
-        return _quantize_nf8(tensor, blocksize)
+        return _quantize_codebook(tensor, "nf8", blocksize)
     if quant_type == "fp8":
         return _quantize_fp(tensor, 8)
     raise ValueError(f"Unknown quantization type: {quant_type}")
@@ -309,27 +291,16 @@ def quantize_nf4_many(tensors, blocksize=64, packed=True):
     ``[quantize_4bit(t, quant_type="nf4", blocksize=blocksize, packed=packed) for t in tensors]``.  One launch per
     tensor: the NF4 code search is latency-bound and its high-occupancy kernel measured faster than the
     multi-tensor TMA stream that serves the affine formats (46.6 vs 64.7 us on 11008 x 4096)."""
-    return [_quantize_nf4(t, blocksize, packed) for t in tensors]
+    return [_quantize_codebook(t, "nf4", blocksize, packed) for t in tensors]
 
 
 def _dequantize_linear(q_tensor, scale, zero_point, blocksize, packed, shape, out_dtype):
-    _host.require_cuda(q_tensor, "q_tensor")
-    dev = q_tensor.device
-    q = q_tensor.detach()
-    if q.dtype != torch.uint8:
-        q = q.to(torch.uint8)
-    if not q.is_contiguous():
-        q = q.contiguous()
+    q = _prep_codes(q_tensor)
+    dev = q.device
     scale = torch.as_tensor(scale, dtype=torch.float32, device=dev).contiguous()
     zp = torch.as_tensor(zero_point, dtype=torch.float32, device=dev).contiguous()
-    if packed:
-        out_shape = torch.Size(shape) if shape is not None else torch.Size([q.numel() * 2])
-    else:
-        out_shape = q.shape
+    out_shape = _out_shape(q, packed, shape)
     n = out_shape.numel()
-    if packed and q.numel() != (n + 1) // 2:
-        # a wrong ``shape`` would make the kernel read past the packed buffer
-        raise ValueError(f"packed codes hold {q.numel()} bytes, shape {tuple(out_shape)} needs {(n + 1) // 2}")
     if n == 0:
         return torch.empty(out_shape, dtype=out_dtype, device=dev)
     ns = scale.numel()
@@ -381,21 +352,11 @@ def _dequantize_many(qs, scales, zero_points, blocksize, packed, shapes, out_dty
     dev = qs[0].device
     cq, cs, cz, ns, out_shapes = [], [], [], [], []
     for q, s, z, shape in zip(qs, scales, zero_points, shapes):
-        _host.require_cuda(q, "q_tensor")
+        q = _prep_codes(q)
         if q.device != dev:
             raise ValueError("all tensors of a batch must share one device")
-        q = q.detach()
-        if q.dtype != torch.uint8:
-            q = q.to(torch.uint8)
-        if not q.is_contiguous():
-            q = q.contiguous()
-        if packed:
-            out_shape = torch.Size(shape) if shape is not None else torch.Size([q.numel() * 2])
-        else:
-            out_shape = q.shape
+        out_shape = _out_shape(q, packed, shape)
         n = out_shape.numel()
-        if packed and q.numel() != (n + 1) // 2:
-            raise ValueError(f"packed codes hold {q.numel()} bytes, shape {tuple(out_shape)} needs {(n + 1) // 2}")
         if n == 0 or n % B:
             raise ValueError(f"numel ({n}) must be a positive multiple of blocksize ({blocksize})")
         s = torch.as_tensor(s, dtype=torch.float32, device=dev).contiguous()
@@ -435,7 +396,7 @@ def dequantize_8bit(q_tensor, scale_or_levels, zero_point_or_bias, quant_type="l
         return _dequantize_linear(q_tensor, scale_or_levels, zero_point_or_bias, blocksize, False, None, out_dtype)
     if quant_type == "nf8":
         # scale_or_levels is the nf8_levels tensor, zero_point_or_bias the abs_max (:39-41)
-        return _dequantize_nf8(q_tensor, zero_point_or_bias, blocksize, out_dtype)
+        return _dequantize_codebook(q_tensor, zero_point_or_bias, "nf8", blocksize, False, None, out_dtype)
     if quant_type == "fp8":
         return _dequantize_fp(q_tensor, zero_point_or_bias, 8, out_dtype)
     raise ValueError(f"Unknown quantization type: {quant_type}")
@@ -450,7 +411,7 @@ def dequantize_4bit(q_tensor, scale_or_levels, zero_point_or_bias, quant_type="l
         return _dequantize_linear(q_tensor, scale_or_levels, zero_point_or_bias, blocksize, packed, shape, out_dtype)
     if quant_type == "nf4":
         # scale_or_levels is the nf4_levels tensor, zero_point_or_bias the abs_max (:59-61)
-        return _dequantize_nf4(q_tensor, zero_point_or_bias, blocksize, packed, shape, out_dtype)
+        return _dequantize_codebook(q_tensor, zero_point_or_bias, "nf4", blocksize, packed, shape, out_dtype)
     if quant_type == "fp4":
         return _dequantize_fp(q_tensor, zero_point_or_bias, 4, out_dtype)
     raise ValueError(f"Unknown quantization type: {quant_type}")

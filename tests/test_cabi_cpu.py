@@ -54,6 +54,16 @@ def test_argument_errors_without_gpu():
     assert h.quanta_quantize_affine(p, 0, 1, 64, 0, 0, 8, 0, p, p, p, p, 16, None) == -3         # workspace
 
 
+def test_nf4_levels_need_no_gpu_and_match_the_oracle():
+    """quanta_nf4_levels copies the library's one NF4 table on the host: no CUDA context, the oracle's bits."""
+    import numpy as np
+    from oracle import oracle_np as O
+    buf = (ctypes.c_float * 16)()
+    assert _lib.lib().quanta_nf4_levels(buf) == 0
+    assert np.array_equal(np.frombuffer(buf, np.float32).view(np.uint32), O.NF4_LEVELS.view(np.uint32))
+    assert _lib.lib().quanta_nf4_levels(None) == -1
+
+
 def test_no_cpu_fallback():
     import quanta_b200 as Q
     from quanta_b200.backends.cuda import quantize_8bit_cuda

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 import torch
 
+from helpers import CODEBOOK_EDGE_CASES, codebook_input
 from oracle import oracle_np as O
 
 pytestmark = pytest.mark.gpu
@@ -52,13 +53,15 @@ def test_nf8_matches_reference_golden():
         assert same_bits(d.cpu().numpy(), Z[f"{c['name']}/deq"]), c
 
 
-@pytest.mark.parametrize("shape,block", [((2048, 1024), None), ((2048, 1024), 64), ((1000, 37), None), ((512, 256), 128)])
-def test_nf8_large_random_matches_oracle(shape, block):
+@pytest.mark.parametrize("shape,block,dtype,case", [
+    pytest.param(shape, block, "float32", None, id=f"shape{i}-{block}")
+    for i, (shape, block) in enumerate([((2048, 1024), None), ((2048, 1024), 64), ((1000, 37), None), ((512, 256), 128)])
+] + CODEBOOK_EDGE_CASES)
+def test_nf8_large_random_matches_oracle(shape, block, dtype, case):
     import quanta_b200 as Q
-    g = torch.Generator().manual_seed(9)
-    x = torch.randn(*shape, generator=g) * 0.02
-    idx, levels, am = Q.quantize_8bit(x.cuda(), quant_type="nf8", blocksize=block)
-    io, ao = O.quantize_nf8(x.numpy(), block)
+    x, xf = codebook_input(shape, dtype, case, seed=9)
+    idx, levels, am = Q.quantize_8bit(x, quant_type="nf8", blocksize=block)
+    io, ao = O.quantize_nf8(xf, block)
     assert np.array_equal(idx.cpu().numpy(), io)
     assert same_bits(am.cpu().numpy(), ao)
     d = Q.dequantize_8bit(idx, levels, am, quant_type="nf8", blocksize=block)

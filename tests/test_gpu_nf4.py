@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 import torch
 
+from helpers import CODEBOOK_EDGE_CASES, codebook_input
 from oracle import oracle_np as O
 
 pytestmark = pytest.mark.gpu
@@ -33,23 +34,26 @@ def test_nf4_matches_reference_golden():
         assert same_bits(d.cpu().numpy(), Z[f"{c['name']}/deq"]), c
 
 
-@pytest.mark.parametrize("shape,block", [((4096, 1024), None), ((4096, 1024), 64), ((1000, 37), None), ((512, 256), 128)])
+@pytest.mark.parametrize("shape,block,dtype,case", [
+    pytest.param(shape, block, "float32", None, id=f"shape{i}-{block}")
+    for i, (shape, block) in enumerate([((4096, 1024), None), ((4096, 1024), 64), ((1000, 37), None), ((512, 256), 128)])
+] + CODEBOOK_EDGE_CASES)
 @pytest.mark.parametrize("packed", [False, True])
-def test_nf4_large_random_matches_oracle(shape, block, packed):
+def test_nf4_large_random_matches_oracle(shape, block, dtype, case, packed):
     import quanta_b200 as Q
-    g = torch.Generator().manual_seed(5)
-    x = torch.randn(*shape, generator=g) * 0.02
-    idx, levels, am = Q.quantize_4bit(x.cuda(), quant_type="nf4", blocksize=block, packed=packed)
-    io, ao = O.quantize_nf4(x.numpy(), block)
+    x, xf = codebook_input(shape, dtype, case, seed=5)
+    idx, levels, am = Q.quantize_4bit(x, quant_type="nf4", blocksize=block, packed=packed)
+    io, ao = O.quantize_nf4(xf, block)
     got = idx.cpu().numpy()
     if packed:
-        got = O.unpack4(got)[: x.numel()].reshape(shape)
+        got = O.unpack4(got)[: xf.size].reshape(shape)
     assert np.array_equal(got, io)
     assert same_bits(am.cpu().numpy(), ao)
     d = Q.dequantize_4bit(idx, levels, am, quant_type="nf4", blocksize=block, packed=packed, shape=shape)
     assert same_bits(d.cpu().numpy(), O.dequantize_nf4(io, ao, block))
-    # size-independent property: every value lands on one of the 16 levels times its abs_max, error <= half a gap
-    assert float((d.cpu() - x).abs().max()) <= 0.16 * float(x.abs().max())
+    if np.isfinite(xf).all():
+        # size-independent property: every value lands on one of the 16 levels times its abs_max, error <= half a gap
+        assert float(np.abs(d.cpu().numpy() - xf).max()) <= 0.16 * float(np.abs(xf).max())
 
 
 @pytest.mark.parametrize("packed", [True, False])
