@@ -319,6 +319,20 @@ QUANTA_API int quanta_gemm_nf4a16_dgrad(const void* dy, int act_dtype, const uin
                              int64_t block, void* dx, int64_t M, int64_t N, int64_t K,
                              void* workspace, size_t workspace_bytes, void* stream);
 
+/* Input gradient of quanta_int8_outlier_matmul (the backward of
+ * Linear8bitLt(outlier_split=True) for a frozen weight), straight-through:
+ *     dx[M,K] = dy[M,N] . W16[N,K],   W16[n,k] = round_act(qw[n,k] / cw[n])
+ * (an IEEE divide, then one rounding to act_dtype): bit for bit the weights
+ * the forward multiplies its outlier columns with.  The threshold, the
+ * outlier set and the int8 quantization of x do not enter.  qw / cw as
+ * passed to the forward; K % 16 == 0.  dy, dx are `act_dtype` (F16 or BF16),
+ * fp32 accumulation; dy rows have a pitch of round_up(N, 8) elements and dx
+ * is [M, K] contiguous.  workspace: quanta_workspace_bytes(QUANTA_OP_GEMM,
+ * M, K), the zero-initialised buffer of quanta_gemm_wna16_dgrad.          */
+QUANTA_API int quanta_int8_outlier_dgrad(const void* dy, int act_dtype, const int8_t* qw, const float* cw, void* dx,
+                              int64_t M, int64_t N, int64_t K,
+                              void* workspace, size_t workspace_bytes, void* stream);
+
 /* LLM.int8()-style outlier-split matmul for Linear8bitLt.threshold
  * (nn/linear.py:20,25; unused by the reference — semantics defined by this
  * repository, see oracle/oracle_np.py:int8_outlier_matmul).

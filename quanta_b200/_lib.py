@@ -56,6 +56,7 @@ SIGNATURES = {
     "quanta_gemm_wna16_dgrad": (_int, [_vp, _int, _vp, _int, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
     "quanta_gemm_nf4a16_dgrad": (_int, [_vp, _int, _vp, _vp, _i64, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
     "quanta_int8_outlier_matmul": (_int, [_vp, _int, _vp, _vp, _f, _vp, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
+    "quanta_int8_outlier_dgrad": (_int, [_vp, _int, _vp, _vp, _vp, _i64, _i64, _i64, _vp, _sz, _vp]),
 }
 
 _lib = None

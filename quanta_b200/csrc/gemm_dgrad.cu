@@ -1,6 +1,9 @@
 // Input gradient of the quantized linear layers on the 5th-generation tensor cores:
 //     dx[M,K] = dy[M,N] . dequant(Wq)[N,K]
-// The weight is frozen, so this is the only gradient the layers need.  It is the forward GEMM
+// The weight is frozen, so this is the only gradient the layers need.  Weight formats: blockwise
+// affine 4/8-bit and NF4 (Linear4bit, Linear8bitLt), and the int8 row-wise codes of the outlier
+// split (ROW8: W16[n,k] = round_act(qw[n,k] / cw[n]), the 16-bit weights of outlier.cu's outlier
+// columns; the straight-through gradient of the LLM.int8() product).  It is the forward GEMM
 // (gemm.cu) with the weight used the other way round: the reduction runs over N (out_features)
 // and the output features are K (in_features).
 //
@@ -21,7 +24,7 @@
 //   warps 8-23  dequantize: 2 groups x 8 warps; group g owns the 64-n blocks g and g + 2 of every
 //               stage (A slots g and g + 2).  Thread -> (code row, quarter of the 128 k): 32 codes
 //               -> 32 16-bit weights with the forward's dequant_word4 / dequant_word8 / NF4 table
-//               -> four 16-byte shared-memory stores into the A slot
+//               (ROW8: dequant_word8_row) -> four 16-byte shared-memory stores into the A slot
 // Work is split stream-K style over (k tile, n stage) units, with the forward's deterministic
 // fix-up, counters and workspace (GemmParams in the OUTPUT's terms: p.N = in_features K is the
 // output width, p.K = out_features N is the reduction length).
@@ -63,7 +66,40 @@ __device__ __forceinline__ void sts128(uint32_t addr, uint32_t a, uint32_t b, ui
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
 }
 
-template <typename ACT, int BITS>
+// int8 row-wise codes (rowwise_quantize_sym): four signed codes -> round_act(q / cw), bit for bit the
+// forward's round_act(__fdiv_rn(q, cw)).  XOR 0x80 makes each byte q + 128, which PRMT drops into
+// 0x4700uu00 = 32768 + q + 128; one add leaves q exactly.  With y = RN(1/cw) hoisted per row,
+// q0 = q y; r = fma(-cw, q0, q); fma(y, r, q0) is the correctly rounded quotient for every code and
+// every cw in [2^-60, 2^60] (affine_quotient's window; exhaustive check: tools/check_rowwise_div.c).
+// Rows outside the window (cw = inf for an all-zero or subnormal row, cw < 2^-60 for a huge one)
+// are redone by dequant_word8_row_div.  Pairs of lanes run as f32x2 FADD2 / FMUL2 / FFMA2.
+__device__ __forceinline__ float2 codes8_row(uint32_t u, int e) {
+    const float2 f = make_float2(__uint_as_float(prmt_(u, 0x47000000u, 0x7504u | ((2 * e) << 4))),
+                                 __uint_as_float(prmt_(u, 0x47000000u, 0x7504u | ((2 * e + 1) << 4))));
+    return __fadd2_rn(f, make_float2(-32896.0f, -32896.0f));
+}
+template <typename ACT>
+__device__ __forceinline__ void dequant_word8_row(uint32_t w, float2 ncw2, float2 y2, uint32_t* out) {
+    const uint32_t u = w ^ 0x80808080u;
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+        const float2 a = codes8_row(u, e);
+        const float2 q0 = __fmul2_rn(a, y2);
+        const float2 q = __ffma2_rn(y2, __ffma2_rn(ncw2, q0, a), q0);
+        out[e] = ActTraits<ACT>::pack(q.x, q.y);
+    }
+}
+template <typename ACT>
+__device__ __forceinline__ void dequant_word8_row_div(uint32_t w, float cw, uint32_t* out) {
+    const uint32_t u = w ^ 0x80808080u;
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+        const float2 a = codes8_row(u, e);
+        out[e] = ActTraits<ACT>::pack(__fdiv_rn(a.x, cw), __fdiv_rn(a.y, cw));
+    }
+}
+
+template <typename ACT, int BITS, bool ROW8>
 __global__ void __launch_bounds__(kDgThreads, 1)
 gemm_dgrad_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_dy,
                   const __grid_constant__ GemmOutputs<1> outs, const float* __restrict__ scale, const float* __restrict__ zp,
@@ -364,7 +400,7 @@ gemm_dgrad_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                 const int n = min(s * kDgRows + (group + 2 * h) * kBlockK + rl, p.K - 1);
                 const int64_t i = (int64_t)n * p.scale_stride + col;
                 sv[h] = __ldg(scale + i);
-                zv[h] = p.nf4 ? 0.0f : __ldg(zp + i);
+                zv[h] = (ROW8 || p.nf4) ? 0.0f : __ldg(zp + i);
             }
         };
         if (a_ok) fetch_params(a_tile, a_s);
@@ -401,6 +437,28 @@ gemm_dgrad_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
                                     uint32_t pr = nf4_pairs[(w4[i] >> (8 * e)) & 0xFFu];
                                     V2 v = __hmul2(*reinterpret_cast<V2*>(&pr), s2);
                                     out[4 * i + e] = *reinterpret_cast<uint32_t*>(&v);
+                                }
+                            }
+                        } else if (ROW8) {
+                            // one multiplier per code row: scale_stride 1, so cs[h] = cw[n]
+                            const float cw = cs[h], y = __frcp_rn(cw);
+                            const float2 y2 = make_float2(y, y), ncw2 = make_float2(-cw, -cw);
+#pragma unroll
+                            for (int g = 0; g < 2; ++g) {
+                                const uint4 rv = lds128g(rrow + (((uint32_t)(2 * q + g) ^ sw) << 4));
+                                dequant_word8_row<ACT>(rv.x, ncw2, y2, out + 8 * g);
+                                dequant_word8_row<ACT>(rv.y, ncw2, y2, out + 8 * g + 2);
+                                dequant_word8_row<ACT>(rv.z, ncw2, y2, out + 8 * g + 4);
+                                dequant_word8_row<ACT>(rv.w, ncw2, y2, out + 8 * g + 6);
+                            }
+                            if (!(cw >= 0x1p-60f && cw <= 0x1p60f)) {
+#pragma unroll
+                                for (int g = 0; g < 2; ++g) {
+                                    const uint4 rv = lds128g(rrow + (((uint32_t)(2 * q + g) ^ sw) << 4));
+                                    dequant_word8_row_div<ACT>(rv.x, cw, out + 8 * g);
+                                    dequant_word8_row_div<ACT>(rv.y, cw, out + 8 * g + 2);
+                                    dequant_word8_row_div<ACT>(rv.z, cw, out + 8 * g + 4);
+                                    dequant_word8_row_div<ACT>(rv.w, cw, out + 8 * g + 6);
                                 }
                             }
                         } else if (BITS == 4) {
@@ -452,7 +510,8 @@ gemm_dgrad_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_const
 
 // ---- host side --------------------------------------------------------------
 
-template <typename ACT, int BITS>
+// ROW8: int8 row-wise codes, `scale` = cw [N], no zero-point, `block` unused
+template <typename ACT, int BITS, bool ROW8 = false>
 static int dgrad_launch(const ACT* dy, const uint8_t* wq, const float* scale, const float* zp, int64_t block, ACT* dx,
                         int64_t M, int64_t N, int64_t K, void* workspace, size_t ws_bytes, cudaStream_t st, int nf4) {
     constexpr uint32_t kRowBytes = kTileN * BITS / 8;
@@ -470,8 +529,8 @@ static int dgrad_launch(const ACT* dy, const uint8_t* wq, const float* scale, co
     p.nbuf = 2;
     p.nf4 = nf4;
     p.n_out = 1; p.ldy = (int)K; p.col0 = 0;
-    p.scale_stride = (int)(K / block);
-    int bs = 0; while ((int64_t)(kBlockK << bs) < block) ++bs;
+    p.scale_stride = ROW8 ? 1 : (int)(K / block);
+    int bs = 0; while (!ROW8 && (int64_t)(kBlockK << bs) < block) ++bs;
     p.block_shift = bs;
     p.vec4 = 0;
 
@@ -525,14 +584,14 @@ static int dgrad_launch(const ACT* dy, const uint8_t* wq, const float* scale, co
     GemmOutputs<1> outs;
     outs.maps[0] = tmap_w;                                   // placeholder
     outs.y[0] = dx;
-    p.vec_store = (reinterpret_cast<uintptr_t>(dx) & 7) == 0 ? 1 : 0;     // K % 64 == 0
+    p.vec_store = (reinterpret_cast<uintptr_t>(dx) & 7) == 0 ? 1 : 0;     // K % 16 == 0
     p.y_tma = (reinterpret_cast<uintptr_t>(dx) & 15) == 0 ? 1 : 0;
     if (p.y_tma) {
         rc = make_tensor_map_2d(&outs.maps[0], ActTraits<ACT>::kTma, 2, dx, (uint64_t)K, (uint64_t)M, (uint64_t)K * 2, kTileN, 16,
                                 CU_TENSOR_MAP_SWIZZLE_NONE);
         if (rc) return rc;
     }
-    auto kern = gemm_dgrad_kernel<ACT, BITS>;
+    auto kern = gemm_dgrad_kernel<ACT, BITS, ROW8>;
     const int smem = (int)(p.x_ring_off + (uint32_t)p.x_stages * p.x_slot_bytes + 1024);
     if (int e = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), smem)) return e;
     const cudaError_t e = launch_pdl(kern, dim3((unsigned)p.G), dim3(kDgThreads), (size_t)smem, st, tmap_w, tmap_dy, outs, scale, zp,
@@ -540,15 +599,21 @@ static int dgrad_launch(const ACT* dy, const uint8_t* wq, const float* scale, co
     return cuda_status(e != cudaSuccess ? e : cudaGetLastError());
 }
 
-// argument checks shared by both entries; all of them run before the first CUDA call
-static int dgrad_check(const void* dy, const uint8_t* wq, const float* scale, const void* dx, int bits, int64_t block,
-                       int64_t M, int64_t N, int64_t K) {
-    if (!dy || !wq || !scale || !dx || M <= 0 || N <= 0 || K <= 0) return QUANTA_EINVAL;
-    if ((bits != 4 && bits != 8) || block <= 0 || block % kBlockK != 0 || K % block != 0) return QUANTA_EINVAL;
-    if ((block / kBlockK) & (block / kBlockK - 1)) return QUANTA_EUNSUPPORTED;          // block = 64 * 2^j
+// argument checks shared by every entry; all of them run before the first CUDA call.  fmt_ok: the
+// entry's weight-format arguments are valid (QUANTA_EINVAL otherwise, like a null pointer).
+static int dgrad_check(const void* dy, const void* wq, const float* scale, const void* dx, bool fmt_ok, int64_t M,
+                       int64_t N, int64_t K) {
+    if (!dy || !wq || !scale || !dx || M <= 0 || N <= 0 || K <= 0 || !fmt_ok) return QUANTA_EINVAL;
     if (M > INT32_MAX || N > INT32_MAX || K > INT32_MAX) return QUANTA_EUNSUPPORTED;
     if ((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(wq)) & 15) return QUANTA_EUNSUPPORTED;
     return QUANTA_OK;
+}
+// blockwise formats: 4 or 8 bits, block = 64 * 2^j dividing K
+static int dgrad_check_block(const void* dy, const uint8_t* wq, const float* scale, const void* dx, int bits,
+                             int64_t block, int64_t M, int64_t N, int64_t K) {
+    const bool fmt_ok = (bits == 4 || bits == 8) && block > 0 && block % kBlockK == 0 && K % block == 0;
+    if (int rc = dgrad_check(dy, wq, scale, dx, fmt_ok, M, N, K)) return rc;
+    return ((block / kBlockK) & (block / kBlockK - 1)) ? QUANTA_EUNSUPPORTED : QUANTA_OK;
 }
 
 }  // namespace quanta
@@ -559,7 +624,7 @@ extern "C" int quanta_gemm_wna16_dgrad(const void* dy, int act_dtype, const uint
                                        const float* zp, int64_t block, void* dx, int64_t M, int64_t N, int64_t K,
                                        void* workspace, size_t workspace_bytes, void* stream) {
     if (!zp) return QUANTA_EINVAL;
-    if (int rc = dgrad_check(dy, wq, scale, dx, bits, block, M, N, K)) return rc;
+    if (int rc = dgrad_check_block(dy, wq, scale, dx, bits, block, M, N, K)) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (act_dtype == QUANTA_BF16) {
         using T = __nv_bfloat16;
@@ -577,7 +642,7 @@ extern "C" int quanta_gemm_wna16_dgrad(const void* dy, int act_dtype, const uint
 extern "C" int quanta_gemm_nf4a16_dgrad(const void* dy, int act_dtype, const uint8_t* wq, const float* absmax, int64_t block,
                                         void* dx, int64_t M, int64_t N, int64_t K, void* workspace, size_t workspace_bytes,
                                         void* stream) {
-    if (int rc = dgrad_check(dy, wq, absmax, dx, 4, block, M, N, K)) return rc;
+    if (int rc = dgrad_check_block(dy, wq, absmax, dx, 4, block, M, N, K)) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     if (act_dtype == QUANTA_BF16) {
         using T = __nv_bfloat16;
@@ -586,6 +651,23 @@ extern "C" int quanta_gemm_nf4a16_dgrad(const void* dy, int act_dtype, const uin
     if (act_dtype == QUANTA_F16) {
         using T = __half;
         return dgrad_launch<T, 4>((const T*)dy, wq, absmax, absmax, block, (T*)dx, M, N, K, workspace, workspace_bytes, st, 1);
+    }
+    return QUANTA_EINVAL;
+}
+
+extern "C" int quanta_int8_outlier_dgrad(const void* dy, int act_dtype, const int8_t* qw, const float* cw, void* dx, int64_t M,
+                                         int64_t N, int64_t K, void* workspace, size_t workspace_bytes, void* stream) {
+    if (int rc = dgrad_check(dy, qw, cw, dx, true, M, N, K)) return rc;
+    if (K % 16 != 0) return QUANTA_EUNSUPPORTED;                                     // TMA row pitch of qw and dx
+    const uint8_t* w = reinterpret_cast<const uint8_t*>(qw);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (act_dtype == QUANTA_BF16) {
+        using T = __nv_bfloat16;
+        return dgrad_launch<T, 8, true>((const T*)dy, w, cw, nullptr, 0, (T*)dx, M, N, K, workspace, workspace_bytes, st, 0);
+    }
+    if (act_dtype == QUANTA_F16) {
+        using T = __half;
+        return dgrad_launch<T, 8, true>((const T*)dy, w, cw, nullptr, 0, (T*)dx, M, N, K, workspace, workspace_bytes, st, 0);
     }
     return QUANTA_EINVAL;
 }

@@ -293,13 +293,7 @@ def int8_outlier_matmul(x, qw, cw, threshold=6.0, bias=None):
     _host.require_cuda(x, "x")
     if x.dtype not in (torch.float16, torch.bfloat16):
         raise TypeError("x must be float16 or bfloat16")
-    if qw.dtype != torch.int8 or qw.dim() != 2:
-        raise TypeError("qw must be an int8 [N, K] tensor")
-    N, K = qw.shape
-    if qw.device != x.device or not qw.is_contiguous():
-        raise ValueError(f"qw must be contiguous and on {x.device}")
-    if not isinstance(cw, torch.Tensor) or cw.dtype != torch.float32 or cw.numel() != N or cw.device != x.device or not cw.is_contiguous():
-        raise TypeError(f"cw must be a contiguous float32 tensor of {N} row multipliers on {x.device}")
+    N, K = _check_rowwise_args(x, qw, cw)
     if x.shape[-1] != K:
         raise ValueError(f"x has {x.shape[-1]} features, weight expects {K}")
     x2 = x.reshape(-1, K)
@@ -320,3 +314,68 @@ def int8_outlier_matmul(x, qw, cw, threshold=6.0, bias=None):
                                                    _host.stream_ptr(dev))
     _lib.check(st, "quanta_int8_outlier_matmul")
     return y.reshape(*x.shape[:-1], N)
+
+
+def _check_rowwise_args(x, qw, cw):
+    """qw int8 [N, K] and cw float32 [N] as the int8 kernels read them; returns (N, K)."""
+    if not isinstance(qw, torch.Tensor) or qw.dtype != torch.int8 or qw.dim() != 2:
+        raise TypeError("qw must be an int8 [N, K] tensor")
+    N, K = qw.shape
+    if qw.device != x.device or not qw.is_contiguous():
+        raise ValueError(f"qw must be contiguous and on {x.device}")
+    if not isinstance(cw, torch.Tensor) or cw.dtype != torch.float32 or cw.numel() != N or cw.device != x.device or not cw.is_contiguous():
+        raise TypeError(f"cw must be a contiguous float32 tensor of {N} row multipliers on {x.device}")
+    return N, K
+
+
+def int8_outlier_dgrad(dy, qw, cw):
+    """dx = dy @ W16 with ``W16[n, k] = round_act(qw[n, k] / cw[n])`` (an IEEE divide, then one rounding to
+    dy's dtype): the input gradient of ``int8_outlier_matmul`` for a frozen weight.  W16 is bit for bit the
+    weight the forward multiplies its outlier columns with, and ``Linear8bitLt.dequantize_weight(dtype)``.
+    The gradient is straight-through: the int8 quantization of x and the outlier set do not enter, so the
+    threshold is not an argument.
+
+    dy [..., N] float16 / bfloat16 (CUDA); qw int8 [N, K] with K % 16 == 0; cw float32 [N].
+    Returns dx [..., K] in dy's dtype (fp32 accumulation)."""
+    _host.require_cuda(dy, "dy")
+    if dy.dtype not in (torch.float16, torch.bfloat16):
+        raise TypeError("dy must be float16 or bfloat16")
+    N, K = _check_rowwise_args(dy, qw, cw)
+    if dy.shape[-1] != N:
+        raise ValueError(f"int8_outlier_dgrad: dy has {dy.shape[-1]} features, weight has {N} outputs")
+    if dy.numel() == 0:
+        return torch.zeros((*dy.shape[:-1], K), dtype=dy.dtype, device=dy.device)
+    dy2, N, K = _dgrad_args(dy, qw, 8, N, K, "int8_outlier_dgrad")
+    M = dy2.shape[0]
+    dev = dy.device
+    dx = torch.empty((M, K), dtype=dy.dtype, device=dev)
+    with _host.device_guard(dev):
+        ws = _host.gemm_workspace(dev, _host.workspace_bytes(_lib.OP_GEMM, M, K))
+        st = _lib.lib().quanta_int8_outlier_dgrad(dy2.data_ptr(), _host.dtype_code(dy2), qw.data_ptr(), cw.data_ptr(),
+                                                  dx.data_ptr(), M, N, K, ws.data_ptr(), ws.numel(), _host.stream_ptr(dev))
+    _lib.check(st, "quanta_int8_outlier_dgrad")
+    return dx.reshape(*dy.shape[:-1], K)
+
+
+class Int8OutlierMatmulFunction(torch.autograd.Function):
+    """``int8_outlier_matmul`` with the straight-through backward for x and bias (bitsandbytes'
+    ``MatMul8bitLt``): ``dx = dy @ W16`` through ``int8_outlier_dgrad``, ``db = dy.sum(0)`` accumulated in fp32.
+    Only qw and cw are saved.  ``bias`` / ``bias_k`` as in ``LinearWNA16Function``; no double backward."""
+
+    @staticmethod
+    def forward(ctx, x, bias, bias_k, qw, cw, threshold):
+        ctx.save_for_backward(qw, cw)
+        ctx.bias_dtype = bias.dtype if bias is not None else None
+        return int8_outlier_matmul(x, qw, cw, threshold, bias_k)
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, dy):
+        qw, cw = ctx.saved_tensors
+        dx = db = None
+        if ctx.needs_input_grad[0]:
+            dx = int8_outlier_dgrad(dy, qw, cw)
+        if ctx.needs_input_grad[1]:
+            db = dy.reshape(-1, qw.shape[0]).sum(0, dtype=torch.float32).to(ctx.bias_dtype)
+        return dx, db, None, None, None, None
+

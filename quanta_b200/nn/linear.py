@@ -13,12 +13,13 @@ bf16/fp16.  ``Linear4bit`` supports ``quant_type="nf4"`` (the reference default:
 blockwise abs_max) and ``quant_type="linear"`` (blockwise affine).
 
 Backward: the quantized weight is frozen (its codes are buffers).  When autograd is recording and x or
-the bias requires a gradient, ``Linear4bit`` and ``Linear8bitLt(outlier_split=False)`` run through an
-autograd Function whose backward gives ``x.grad = dy @ W`` (the fused dequantize-transposed GEMM,
-with bit-for-bit the weights of the forward) and ``bias.grad = dy.sum(0)`` (fp32 accumulation).  The
-forward launches the same kernel with the same arguments either way.  Not differentiable: the
-outlier split (``outlier_split=True``), the tensor-parallel layers, the weight itself, and a double
-backward.
+the bias requires a gradient, ``Linear4bit`` and ``Linear8bitLt`` run through an autograd Function whose
+backward gives ``x.grad = dy @ W`` (the fused dequantize-transposed GEMM, with bit-for-bit the weights of
+the forward) and ``bias.grad = dy.sum(0)`` (fp32 accumulation).  The forward launches the same kernel with
+the same arguments either way.  With ``outlier_split=True`` the gradient is the straight-through one of
+the LLM.int8() product (bitsandbytes' ``MatMul8bitLt``): W is ``dequantize_weight(dtype)``, i.e.
+``round_act(qw / row_scale)``, and the threshold, the outlier columns and the int8 quantization of x do
+not enter.  Not differentiable: the tensor-parallel layers, the weight itself, and a double backward.
 """
 from __future__ import annotations
 
@@ -29,7 +30,7 @@ import torch.nn as nn
 
 from ..functional.quantization import quantize_4bit, quantize_8bit, dequantize_4bit, dequantize_8bit
 from .functional import (linear_wna16, linear_nf4a16, int8_outlier_matmul, rowwise_quantize_sym, LinearWNA16Function,
-                         LinearNF4A16Function)
+                         LinearNF4A16Function, Int8OutlierMatmulFunction)
 
 
 _QUANT_BUFFERS = ("qweight", "scale", "zero_point", "qweight_rowwise", "row_scale")
@@ -182,8 +183,10 @@ class Linear8bitLt(_QuantLinearBase):
     codes, int8 x int8 tensor-core product for the regular feature columns and
     a 16-bit product for the columns whose activations exceed ``threshold``.
 
-    Differentiable in x and bias with ``outlier_split=False`` (module docstring); the outlier split
-    is inference-only."""
+    Differentiable in x and bias in both modes (module docstring).  With ``outlier_split=True`` the
+    backward is straight-through: ``x.grad = dy @ dequantize_weight(dtype)``, the 16-bit weights the
+    forward uses for its outlier columns, whatever the threshold selected; the 8-bit LoRA setting of a
+    frozen int8 base under trainable adapters gets the base's ``dy @ W`` term in ``x.grad``."""
     bits = 8
 
     def __init__(self, in_features, out_features, bias=True, has_fp16_weights=False, threshold=6.0, blocksize=64,
@@ -219,7 +222,11 @@ class Linear8bitLt(_QuantLinearBase):
                 raise RuntimeError("quanta_b200 layers run on CUDA only: move the module to a GPU first")
             self.quantize_()
         xin = x if x.dtype == dt else x.to(dt)
-        y = int8_outlier_matmul(xin, self.qweight_rowwise, self.row_scale, self.threshold, self._bias_as(dt, x.device))
+        if self._records_grad(xin):
+            y = Int8OutlierMatmulFunction.apply(xin, self.bias, self._bias_as(dt, x.device), self.qweight_rowwise,
+                                                self.row_scale, self.threshold)
+        else:
+            y = int8_outlier_matmul(xin, self.qweight_rowwise, self.row_scale, self.threshold, self._bias_as(dt, x.device))
         return y if y.dtype == x.dtype or not x.is_floating_point() else y.to(x.dtype)
 
 
